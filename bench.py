@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — kriged target locations per second (mean + variance), BASELINE.json's metric.
 
-    python bench.py --gpus N --steps K --warmup W [--config C5] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--config C5] [--impl reference] [--dump-outputs DIR]
 
 The headline workload is BASELINE.json's multi-GPU configuration, **C5** (local Ordinary Kriging,
 Spherical variogram, maxneighbors = 64, 1e6 3-D samples onto the 512^3 grid), at every N with **strong
@@ -22,6 +22,11 @@ O(n^2)) are measured in the same run, sharded over the same N ranks, with fewer 
 fraction. `--config X` makes X the headline instead (and `--no-secondary` skips the block).
 
 The CPU oracle is used only for the `cpu_baseline` / `--impl reference` legs.
+
+`--dump-outputs DIR` writes what the headline's last timed step computed, as a caller of that path receives it (the
+whole job; on N > 1 the gathered job), to DIR/target.npy (linear grid index of each value), DIR/mean.npy and
+DIR/variance.npy, all float64. A job larger than DUMP_BYTES is represented by a fixed, seeded sample of DUMP_SAMPLE
+targets. The inputs are synthetic and seeded, so two builds run with the same arguments can be compared value for value.
 """
 from __future__ import annotations
 
@@ -48,6 +53,9 @@ HEADLINE = "C5"
 ALL_CONFIGS = ["C1", "C2", "C3a", "C3b", "C4", "C5"]
 SECONDARY = ["C2", "C3a", "C3b", "C4"]
 C4_BATCH = 262_144          # targets of C4 computed per step (the full 2048^2 grid is 16 such batches)
+DUMP_BYTES = 64 << 20       # --dump-outputs: at most this much in all (three float64 arrays)
+DUMP_SAMPLE = 1 << 20       # targets written for a job larger than that
+DUMP_SEED = 0
 
 
 def host_cores() -> int:
@@ -314,18 +322,40 @@ class Workload:
         env, torch = self.env, self.env.torch
         sampler = ClockSampler(env.local_rank) if (sampler_rank0 and env.rank == 0) else None
         evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
-        env.barrier()
-        wall0 = time.perf_counter()
-        for a, b in evs:
-            env.flush.zero_()
-            a.record(env.stream)
-            self.step()
-            b.record(env.stream)
-        env.barrier()
-        wall = time.perf_counter() - wall0
-        clocks = sampler.stop() if sampler else None
+        try:
+            env.barrier()
+            wall0 = time.perf_counter()
+            for a, b in evs:
+                env.flush.zero_()
+                a.record(env.stream)
+                self.step()
+                b.record(env.stream)
+            env.barrier()
+            wall = time.perf_counter() - wall0
+        finally:                                          # a failing step must not leave nvidia-smi polling
+            clocks = sampler.stop() if sampler else None
         dev_ms = env.max_over_ranks(sum(a.elapsed_time(b) for a, b in evs))
         return dev_ms / steps, wall, clocks
+
+    def dump_outputs(self, out_dir):
+        """mean and variance of the job as the last step left them (see --dump-outputs), on the rank that calls it"""
+        torch, (jf, jc) = self.env.torch, self.job
+        if self.hdl is not None:
+            mean, var = self.sbuf[:jc], self.sbuf[jc:]
+        elif self.env.world > 1:
+            mean, var = self.g_mean, self.g_var
+        else:
+            mean, var = self.d_mean, self.d_var
+        if 3 * 8 * jc <= DUMP_BYTES:
+            pick = np.arange(jc, dtype=np.int64)
+        else:
+            pick = np.sort(np.random.default_rng(DUMP_SEED).choice(jc, DUMP_SAMPLE, replace=False))
+        sel = torch.from_numpy(pick).to(self.env.dev)
+        out = Path(out_dir)
+        out.mkdir(parents=True, exist_ok=True)
+        np.save(out / "target.npy", (jf + pick).astype(np.float64))
+        np.save(out / "mean.npy", mean.index_select(0, sel).cpu().numpy())
+        np.save(out / "variance.npy", var.index_select(0, sel).cpu().numpy())
 
     def check_gather(self):
         """the gathered field must be identical on every rank and hold this rank's slab at its place"""
@@ -532,7 +562,7 @@ def measure_callers(env: Env):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of the headline config")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default=HEADLINE, choices=ALL_CONFIGS)
@@ -543,7 +573,13 @@ def main():
     ap.add_argument("--gather", default="multicast", choices=["peer", "multicast", "nccl"],
                     help="N>1 result gather: stores into every rank's symmetric-memory buffer fused in the solve kernel "
                          "(peer), the same through one NVLS multicast store (multicast), or an NCCL all-gather (nccl)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline's last timed step (target index, mean, variance) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the product path's outputs; the reference arm times a calibrated CPU sample")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -560,6 +596,8 @@ def main():
 
     ms_per_step, wall, clocks = w.timed_steps(args.steps, sampler_rank0=True)
     value = w.job[1] / (ms_per_step * 1e-3)
+    if args.dump_outputs and env.rank == 0:              # before any later leg overwrites the step's buffers
+        w.dump_outputs(args.dump_outputs)
     w.check_gather()
 
     long_step = ms_per_step > 1000.0
