@@ -19,7 +19,13 @@ SIMPLE, ORDINARY, UNIVERSAL = 0, 1, 2
 
 
 def variogram(kind, h, rng, sill, nugget, eps=1e-6):
-    h = np.asarray(h, dtype=np.float64)
+    """γ(h) in the precision of h: float64, or np.longdouble for the extended reference (extended_ref.py). The model
+    constants are converted first, so that sill − nugget − ε is formed in that precision too (in float64 it rounds,
+    and the rounding would reach every covariance sill − γ as a constant offset)."""
+    h = np.asarray(h)
+    h = h.astype(np.result_type(h.dtype, np.float64), copy=False)
+    f = h.dtype.type
+    rng, sill, nugget, eps = f(rng), f(sill), f(nugget), f(eps)
     if kind == GAUSSIAN:
         n = nugget + eps
         g = (sill - n) * (1.0 - np.exp(-3.0 * (h / rng) ** 2))

@@ -116,11 +116,16 @@ def test_target_order_is_visiting_order(gsk, ctx, oracle):
 
 
 # ---- values-only update / plan reuse ----
-@pytest.mark.parametrize("shape", ["local_grid", "local_points", "global"])
+@pytest.mark.parametrize("shape", ["local_grid", "local_points", "global", "global_sk", "global_uk2"])
 def test_update_values_equals_fresh_call(gsk, shape):
     rng = np.random.default_rng(11)
-    if shape == "global":
+    if shape.startswith("global"):
         spec = gsk.synth.config_spec("C1", grid=(30, 30), n=200)
+        if shape != "global":   # the SK value column holds z − μ; UK2 refines 6 drift weights
+            est, deg = (gsk.EST_SIMPLE, 0) if shape == "global_sk" else (gsk.EST_UNIVERSAL, 2)
+            spec = gsk.ProblemSpec(coords=spec.coords, values=spec.values, grid_dims=spec.grid_dims,
+                                   support=spec.support, **dict(spec.params, estimator=est, uk_degree=deg,
+                                                                sk_mean=float(spec.values.mean())))
     else:
         spec = gsk.synth.config_spec("C3a", scale=0.08)
         if shape == "local_points":
@@ -148,7 +153,7 @@ def test_update_values_equals_fresh_call(gsk, shape):
         second = c.timing()
         assert np.array_equal(d_mean.cpu().numpy(), want_mean, equal_nan=True)
         assert np.array_equal(d_var.cpu().numpy(), want_var, equal_nan=True)
-        if shape != "global":
+        if not shape.startswith("global"):
             assert second["launches"] < first["launches"]            # the search (and the bin sort) was skipped
         with pytest.raises(gsk.GskError):
             c.update_values(new_vals[:-1])

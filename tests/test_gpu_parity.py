@@ -149,7 +149,12 @@ def test_matrix(gsk, ctx, oracle, dim, vk, est, deg):
                            vario_kind=vk, vario_range=rng, vario_sill=1.3, vario_nugget=0.05, estimator=est,
                            uk_degree=deg, sk_mean=float(vals.mean()), max_neighbors=k)
     loose = vk == 0 or (est == 2 and deg == 2)    # Gaussian / quadratic drift in raw coordinates: cond ≳ 1e6
-    _check(gsk, ctx, oracle, spec, **(dict(atol_mean=1e-7, atol_var=1e-7) if loose else {}))
+    mean, var = _check(gsk, ctx, oracle, spec, **(dict(atol_mean=1e-7, atol_var=1e-7) if loose else {}))
+    if est == 1:   # k <= 20: the small kernel; UK of degree 0 is Ordinary Kriging bit for bit
+        uk0 = gsk.ProblemSpec(coords=spec.coords, values=spec.values, grid_dims=grid, support=spec.support,
+                              **dict(spec.params, estimator=2, uk_degree=0))
+        m0, v0 = ctx.krige(uk0)
+        assert np.array_equal(m0, mean, equal_nan=True) and np.array_equal(v0, var, equal_nan=True)
 
 
 # ---- edge cases ----
@@ -600,3 +605,79 @@ def test_block_pool_matrix(gsk, ctx, oracle, k, vk, nugget, dim, est, deg):
                            ball_radius=float("nan") if radius is None else radius)
     loose = vk == 0 or deg == 2 or (est == 2 and k >= 40)   # Gaussian / drift monomials in raw coordinates: cond ≳ 1e6
     _check(gsk, ctx, oracle, spec, **(dict(atol_mean=2e-7, atol_var=2e-7) if loose else {}))
+
+
+# ---- the column-packed kernel where only it runs: configuration D (3-D UK2, 25 <= k <= 56) and E (64 < k <= 96, or
+# more than 6 drift terms above k = 56) — the two configurations on the bottom-up row layout (RS % G != 0) ----
+def _colpack_cases():
+    cases = [(3, 2, 2, k, i % 3, (i // 3) % 2) for i, k in enumerate((25, 29, 32, 33, 40, 48, 49, 56, 57, 64))]
+    for a, k in enumerate((65, 66, 72, 73, 80, 88, 89, 95, 96)):   # dimension × variogram: every pair over the ks
+        cases += [((a + j) % 3 + 1 if deg < 2 else 2, est, deg, k, (a + 2 * j) % 3, (a + j) % 2)
+                  for j, (est, deg) in enumerate(((0, 0), (1, 0), (2, 1), (2, 2)))]
+    return [(dim, est, deg, k, vk, (0.0, 0.07)[g]) for dim, est, deg, k, vk, g in cases]
+
+
+COLPACK = _colpack_cases()
+# Every combination above fits the 227 KB of shared memory per CTA (the support offsets move to global memory when they
+# do not): the largest, E with 12 extra rows in 3-D, needs 231 712 bytes of 232 448 — so none answers
+# GSK_ERR_UNSUPPORTED, and the test fails if one does.
+COLPACK_UNSUPPORTED = ()
+
+
+def colpack_spec(gsk, dim, est, deg, k, vk, nugget):
+    grid = {1: (300,), 2: (17, 13), 3: (8, 7, 6)}[dim]
+    n = {1: 300, 2: 520, 3: 800}[dim]
+    coords, vals = gsk.synth.make_samples(700 + dim, n, grid, seed_extra=k + 7 * vk + 3 * est + deg)
+    rng_ = {1: 30.0, 2: 11.0, 3: 7.0}[dim]
+    dens = n / np.prod(grid)
+    knn_r = {1: k / (2 * dens), 2: np.sqrt(k / (np.pi * dens)), 3: (k / (4.18879 * dens)) ** (1 / 3)}[dim]
+    c = 0 if est == 0 else (1 if est == 1 else len(gsk.uk_exponents(deg, dim)))
+    return gsk.ProblemSpec(coords=coords, values=vals, grid_dims=grid, support=gsk.default_support_py([1.0] * dim, rng_),
+                           vario_kind=vk, vario_range=rng_, vario_sill=1.2, vario_nugget=nugget, estimator=est,
+                           uk_degree=deg, sk_mean=float(vals.mean()), max_neighbors=k, min_neighbors=max(3, c + 10),
+                           ball_radius=0.95 * knn_r if k % 8 == 0 else float("nan"))
+
+
+def colpack_reference_rows(nn, k, mean):
+    """≤ 32 targets: up to 16 with a partly filled list (ball), the rest full; none missing."""
+    rng = np.random.default_rng(k)
+    ok = ~np.isnan(mean)
+    part, full = np.flatnonzero(ok & (nn < k)), np.flatnonzero(ok & (nn == k))
+    part = rng.choice(part, min(16, part.size), replace=False)
+    return np.sort(np.concatenate([part, rng.choice(full, min(32 - part.size, full.size), replace=False)]))
+
+
+@pytest.mark.parametrize("dim,est,deg,k,vk,nugget", COLPACK,
+                         ids=[f"d{c[0]}-e{c[1]}{c[2]}-k{c[3]}-v{c[4]}-g{c[5]}" for c in COLPACK])
+def test_column_packed_matrix(gsk, ctx, oracle, dim, est, deg, k, vk, nugget):
+    """Configurations D and E of local_solve.cuh against the oracle (neighbour lists bit-exact, parity rule on every
+    target) and, on up to 32 targets, against the extended-precision reference at |gpu − ref| ≤ c·u·B + 2u·|ref|,
+    c = 4(m + q) (derivation: tests/test_gpu_global_reference.py, oracle/extended_ref.py). For spherical and exponential
+    variograms that bound must itself be below 1e-10 (relative to max(1, |z|), resp. the sill). k % 8 == 0 adds a ball
+    just inside the k-NN radius, so some targets solve with fewer than k neighbours and some are missing."""
+    import extended_ref as XR
+    spec = colpack_spec(gsk, dim, est, deg, k, vk, nugget)
+    if (dim, est, deg, k) in COLPACK_UNSUPPORTED:
+        with pytest.raises(gsk.GskError) as err:
+            ctx.krige(spec)
+        assert err.value.code == -2
+        return
+    (mean, var, nn, idx), (om, ov, onn, oidx) = _both(ctx, oracle, spec)
+    assert np.array_equal(nn, onn) and np.array_equal(idx, oidx)
+    scale = max(1.0, np.abs(spec.values).max())
+    loose = vk == 0 or deg == 2 or (est == 2 and k >= 40)   # as the block-pool matrix: cond ≳ 1e6
+    assert_parity(mean, var, om, ov, scale=scale, sill=1.2, **(dict(atol_mean=2e-7, atol_var=2e-7) if loose else {}))
+    if k % 8 == 0:
+        assert (nn < k).any()
+    rows = colpack_reference_rows(nn, k, om)
+    ref = XR.reference(spec, rows, oidx, onn)
+    tm, tv = ref.tolerances(4)
+    if vk != 0:
+        assert tm.max() <= 1e-10 * scale and tv.max() <= 1e-10 * 1.2
+    assert np.all(np.abs(mean[rows] - ref.mean) <= tm), np.max(np.abs(mean[rows] - ref.mean) / tm)
+    assert np.all(np.abs(var[rows] - ref.var) <= tv), np.max(np.abs(var[rows] - ref.var) / tv)
+    if est == 1:   # the column-packed c == 1 branch: UK of degree 0 is Ordinary Kriging bit for bit
+        uk0 = gsk.ProblemSpec(coords=spec.coords, values=spec.values, grid_dims=spec.grid_dims, support=spec.support,
+                              **dict(spec.params, estimator=2, uk_degree=0))
+        m0, v0 = ctx.krige(uk0)
+        assert np.array_equal(m0, mean, equal_nan=True) and np.array_equal(v0, var, equal_nan=True)
