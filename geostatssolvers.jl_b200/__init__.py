@@ -16,7 +16,8 @@ from .host import (CartesianGrid, EstimationProblem, Euclidean, ExponentialVario
                    GaussianVariogram, GeoTable, IDWSolver, K, KBallSearch, KNearestSearch, Kriging, KrigingSolver, LWRSolver,
                    LinearPath, MetricBall, MultiGridPath, NoUnits, OrdinaryKriging, PointSet, Quantities, RandomPath,
                    SimpleKriging, SphericalVariogram, UniversalKriging, Unit, UnsupportedOption, approxsolve, asarray,
-                   default_context, degC, elunit, embeddim, exactsolve, georef, kriging_ui, maxneighbors, nelements,
+                   default_context, degC, elunit, embeddim, exactsolve, georef, kriging_ui, leave_one_out, maxneighbors,
+                   nelements,
                    preprocess, searcher_ui, solve, traverse, uadjust)
 from . import sharding, simulation, synth  # noqa: F401
 from .simulation import FFTGS, LUGS, SGS, SimulationProblem  # noqa: F401

@@ -214,6 +214,20 @@ class ProblemSpec:
         return p
 
 
+def loo_struct(spec: ProblemSpec) -> GskProblem:
+    """The ``GskProblem`` of a leave-one-out call: the spec's samples and parameters, no targets of its own (the
+    samples are the targets), point support."""
+    p = spec.c_struct()
+    p.grid_dims[0] = 0
+    p.n_points = 0
+    p.n_support = 1
+    for d in range(3):
+        p.point_coords[d] = None
+        p.support_offsets[d] = None
+    p.target_order = None
+    return p
+
+
 # ------------------------------------------------------------------------------------
 # library loading
 # ------------------------------------------------------------------------------------
@@ -251,6 +265,8 @@ def load_library(path: os.PathLike | None = None):
     lib.gsk_synchronize.restype = C.c_int
     lib.gsk_krige.argtypes = [ctx, pp, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.gsk_krige.restype = C.c_int
+    lib.gsk_krige_loo.argtypes = [ctx, pp, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.gsk_krige_loo.restype = C.c_int
     lib.gsk_krige_multi.argtypes = [_ip, C.c_int, pp, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_char_p, C.c_int]
     lib.gsk_krige_multi.restype = C.c_int
     lib.gsk_krige_multi_release.argtypes = []
@@ -298,7 +314,7 @@ def load_library(path: os.PathLike | None = None):
 
 
 EXPORTED_SYMBOLS = [
-    "gsk_create", "gsk_destroy", "gsk_last_error", "gsk_set_stream", "gsk_synchronize", "gsk_krige", "gsk_krige_multi", "gsk_krige_multi_release", "gsk_plan",
+    "gsk_create", "gsk_destroy", "gsk_last_error", "gsk_set_stream", "gsk_synchronize", "gsk_krige", "gsk_krige_loo", "gsk_krige_multi", "gsk_krige_multi_release", "gsk_plan",
     "gsk_execute", "gsk_execute_peers", "gsk_update_values", "gsk_lu_plan", "gsk_lu_sample", "gsk_sgs_plan", "gsk_sgs_sample", "gsk_sgs_sample_device", "gsk_sgs_weights", "gsk_get_timing", "gsk_set_phase_timing", "gsk_num_targets", "gsk_uk_exponents", "gsk_default_support",
     "gsk_measure_fp64_peak", "gsk_abi_version",
 ]
@@ -349,6 +365,31 @@ class Context:
         rc = self.lib.gsk_krige(self._h, C.byref(ps), mean.ctypes.data, var.ctypes.data,
                                 nneigh.ctypes.data if nneigh is not None else None,
                                 idx.ctypes.data if idx is not None else None)
+        self._check(rc)
+        if want_neighbors:
+            return mean, var, nneigh, idx
+        if want_nneigh:
+            return mean, var, nneigh
+        return mean, var
+
+    def krige_loo(self, spec: ProblemSpec, want_nneigh: bool = False, want_neighbors: bool = False):
+        """Leave-one-out cross-validation of the spec's samples (``gsk_krige_loo``): row i is sample i kriged at point
+        support from the other samples. The spec's targets and support are not used (the samples are the targets);
+        its slab (target_first, target_count) counts sample indices."""
+        n = spec.n_samples
+        first = spec.target_first
+        count = n - first if spec.target_count < 0 else spec.target_count
+        if not (0 <= first and 0 <= count and first + count <= n):
+            raise ValueError("sample slab out of range")
+        mean = np.empty(count, dtype=np.float64)
+        var = np.empty(count, dtype=np.float64)
+        k = spec.params["max_neighbors"]
+        nneigh = np.empty(count, dtype=np.int32) if (want_neighbors or want_nneigh) else None
+        idx = np.empty((count, max(k, 1)), dtype=np.int32) if (want_neighbors and k > 0) else None
+        ps = loo_struct(spec)
+        rc = self.lib.gsk_krige_loo(self._h, C.byref(ps), mean.ctypes.data, var.ctypes.data,
+                                    nneigh.ctypes.data if nneigh is not None else None,
+                                    idx.ctypes.data if idx is not None else None)
         self._check(rc)
         if want_neighbors:
             return mean, var, nneigh, idx

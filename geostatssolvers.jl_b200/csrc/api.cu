@@ -559,8 +559,21 @@ static int execute_impl(gsk_ctx *ctx, int64_t first, int64_t count, int32_t *d_n
     return gsk_launch_simple_solver(ctx, st, f, c, nn, nbr, off, nullptr, &launches);
   };
   if (ctx->prob.max_neighbors == 0) {
-    if (kriging) rc = gsk_global_execute(ctx, first, count, d_nneigh, &launches);
-    else rc = gsk_launch_simple_solver(ctx, ctx->stream, first, count, nullptr, nullptr, 0, d_nneigh, &launches);
+    if (ctx->loo) {
+      if (phase_timing) cudaEventRecord(ctx->ev[4], ctx->stream);
+      rc = gsk_global_loo(ctx, first, count, d_nneigh, &launches);
+      if (rc == GSK_OK && phase_timing) {
+        cudaEventRecord(ctx->ev[5], ctx->stream);
+        cudaEventSynchronize(ctx->ev[5]);
+        float b2 = 0.f;
+        cudaEventElapsedTime(&b2, ctx->ev[4], ctx->ev[5]);
+        ms_solve += b2;
+      }
+    } else if (kriging) {
+      rc = gsk_global_execute(ctx, first, count, d_nneigh, &launches);
+    } else {
+      rc = gsk_launch_simple_solver(ctx, ctx->stream, first, count, nullptr, nullptr, 0, d_nneigh, &launches);
+    }
     if (rc != GSK_OK) return rc;
   } else if (!ctx->tg.is_grid && count > 0) {
     // explicit points: process the slab in bin-sorted order (spatially coherent CTAs), then scatter back
@@ -568,7 +581,8 @@ static int execute_impl(gsk_ctx *ctx, int64_t first, int64_t count, int32_t *d_n
     int *perm = nullptr, *nn_s = nullptr, *nbr_s = nullptr;
     double *sx = nullptr, *sy = nullptr, *sz = nullptr, *ms = nullptr, *vs = nullptr;
     // after a values-only update the bin order and the neighbour lists of the same range are still valid
-    const bool reuse = ctx->nbr_reuse && ctx->nbr_cached && ctx->nbr_first == first && ctx->nbr_count == count && ctx->pt_perm;
+    const bool reuse = !ctx->loo && ctx->nbr_reuse && ctx->nbr_cached && ctx->nbr_first == first && ctx->nbr_count == count &&
+                       ctx->pt_perm;
     if (reuse) {
       perm = ctx->pt_perm; sx = ctx->pt_sx; sy = ctx->pt_sy; sz = ctx->pt_sz;
     } else {
@@ -588,13 +602,23 @@ static int execute_impl(gsk_ctx *ctx, int64_t first, int64_t count, int32_t *d_n
     ctx->out.mean[0] = ms;
     ctx->out.var[0] = vs;
     if (phase_timing) cudaEventRecord(ctx->ev[3], ctx->stream);
-    if (!reuse) rc = gsk_launch_search(ctx, ctx->stream, 0, count, nn_s, nbr_s, &launches);
+    if (ctx->loo) {
+      // leave-one-out: the k+1 nearest in the exact (d², index) order contain the k nearest j != i, so search one more
+      // and drop the target's own index (k + 1 <= n_samples: validate_loo)
+      rc = ensure(ctx, (void **)&ctx->d_nn, &ctx->cap_nn, sizeof(int) * (size_t)count);
+      if (rc == GSK_OK) rc = ensure(ctx, (void **)&ctx->d_nbr, &ctx->cap_nbr, sizeof(int) * (size_t)count * (k + 1));
+      if (rc == GSK_OK) rc = gsk_launch_search(ctx, ctx->stream, 0, count, k + 1, ctx->d_nn, ctx->d_nbr, &launches);
+      if (rc == GSK_OK) rc = gsk_points_loo_compact(ctx, perm, first, count, k, ctx->d_nn, ctx->d_nbr, nn_s, nbr_s);
+      ++launches;
+    } else if (!reuse) {
+      rc = gsk_launch_search(ctx, ctx->stream, 0, count, k, nn_s, nbr_s, &launches);
+    }
     if (phase_timing) cudaEventRecord(ctx->ev[4], ctx->stream);
     if (rc == GSK_OK) rc = launch_body(ctx->stream, 0, count, nn_s, nbr_s, 0);
     ctx->tg = tg_saved;
     ctx->out = out_saved;
     if (rc != GSK_OK) return rc;
-    ctx->nbr_cached = true;
+    ctx->nbr_cached = !ctx->loo;  // leave-one-out lists belong to no problem a later gsk_execute could plan
     ctx->nbr_first = first; ctx->nbr_count = count;
     ctx->pt_perm = perm; ctx->pt_sx = sx; ctx->pt_sy = sy; ctx->pt_sz = sz;
     if (phase_timing) {
@@ -645,7 +669,7 @@ static int execute_impl(gsk_ctx *ctx, int64_t first, int64_t count, int32_t *d_n
       int *nbr = d_neigh_idx ? d_neigh_idx + off * k : ctx->d_nbr + (keep ? (size_t)off * k : 0);
       if (phase_timing) cudaEventRecord(ctx->ev[3], ctx->stream);
       if (!reuse) {
-        rc = gsk_launch_search(ctx, ctx->stream, first + off, cnt, nn, nbr, &launches);
+        rc = gsk_launch_search(ctx, ctx->stream, first + off, cnt, k, nn, nbr, &launches);
         if (rc != GSK_OK) return rc;
       }
       if (phase_timing) cudaEventRecord(ctx->ev[4], ctx->stream);
@@ -973,6 +997,62 @@ extern "C" GSK_API int gsk_krige(gsk_ctx *ctx, const gsk_problem *p, double *mea
 } catch (const std::exception &e) {
   if (ctx) { cudaStreamSynchronize(ctx->stream2); cudaStreamSynchronize(ctx->stream); }
   return fail(ctx, GSK_ERR_STATE, std::string("gsk_krige: ") + e.what());
+}
+
+// ---------------------------------------------------------------------------------------------
+// leave-one-out cross-validation: the samples are the targets, each kriged without itself
+// ---------------------------------------------------------------------------------------------
+static int validate_loo(gsk_ctx *ctx, const gsk_problem *p) {
+  if (!p) return fail(ctx, GSK_ERR_INVALID, "problem is NULL");
+  if (p->abi_version != GSK_ABI_VERSION) return fail(ctx, GSK_ERR_INVALID, "gsk_problem.abi_version mismatch");
+  if (p->solver != GSK_SOLVER_KRIGING)
+    return fail(ctx, GSK_ERR_UNSUPPORTED, "gsk_krige_loo: leave-one-out is implemented for the Kriging solver only");
+  if (p->grid_dims[0] != 0 || p->n_points != 0 || p->target_order)
+    return fail(ctx, GSK_ERR_INVALID, "gsk_krige_loo: the targets are the samples (grid_dims[0] = 0, n_points = 0, "
+                                      "target_order = NULL)");
+  if (p->n_support != 1) return fail(ctx, GSK_ERR_INVALID, "gsk_krige_loo: point support only (n_support = 1)");
+  for (int d = 0; d < 3; ++d)
+    if (p->support_offsets[d] && p->support_offsets[d][0] != 0.0)
+      return fail(ctx, GSK_ERR_INVALID, "gsk_krige_loo: the support offset must be zero");
+  if (p->flags & GSK_FLAG_REUSE_PLAN)
+    return fail(ctx, GSK_ERR_INVALID, "gsk_krige_loo: GSK_FLAG_REUSE_PLAN does not apply (no plan is kept)");
+  if (p->n_samples < 2) return fail(ctx, GSK_ERR_INVALID, "gsk_krige_loo: n_samples must be >= 2");
+  if (p->max_neighbors > p->n_samples - 1)
+    return fail(ctx, GSK_ERR_INVALID, "gsk_krige_loo: max_neighbors must be clamped to n_samples - 1 by the host (each "
+                                      "fold holds n_samples - 1 samples)");
+  const int64_t first = p->target_first, count = p->target_count < 0 ? p->n_samples - first : p->target_count;
+  if (first < 0 || count < 0 || first + count > p->n_samples)
+    return fail(ctx, GSK_ERR_INVALID, "gsk_krige_loo: sample slab out of range");
+  return GSK_OK;
+}
+
+extern "C" GSK_API int gsk_krige_loo(gsk_ctx *ctx, const gsk_problem *p, double *mean_out, double *var_out,
+                                     int32_t *nneigh_out, int32_t *neigh_idx_out) try {
+  if (!ctx) return GSK_ERR_INVALID;
+  if (!mean_out || !var_out) return fail(ctx, GSK_ERR_INVALID, "mean_out / var_out are NULL");
+  int rc = validate_loo(ctx, p);
+  if (rc != GSK_OK) return rc;
+  // the explicit point list of the plan is the sample coordinates themselves: target t is sample t
+  gsk_problem q = *p;
+  q.n_points = p->n_samples;
+  for (int d = 0; d < 3; ++d) q.point_coords[d] = p->coords[d];
+  rc = gsk_plan(ctx, &q);
+  if (rc == GSK_OK) {
+    const int64_t first = p->target_first, count = p->target_count < 0 ? p->n_samples - first : p->target_count;
+    ctx->loo = true;
+    if (count > 0) rc = krige_pieces(ctx, &q, first, count, mean_out, var_out, nneigh_out, neigh_idx_out);
+    ctx->loo = false;
+  }
+  // nothing of the leave-one-out plan (sample-target bins order, self-excluded lists) may serve a later gsk_execute
+  cudaStreamSynchronize(ctx->stream);
+  free_plan(ctx);
+  return rc;
+} catch (const std::bad_alloc &) {  // no exception may cross the C ABI
+  if (ctx) { ctx->loo = false; cudaStreamSynchronize(ctx->stream2); cudaStreamSynchronize(ctx->stream); free_plan(ctx); }
+  return fail(ctx, GSK_ERR_NOMEM, "gsk_krige_loo: out of host memory");
+} catch (const std::exception &e) {
+  if (ctx) { ctx->loo = false; cudaStreamSynchronize(ctx->stream2); cudaStreamSynchronize(ctx->stream); free_plan(ctx); }
+  return fail(ctx, GSK_ERR_STATE, std::string("gsk_krige_loo: ") + e.what());
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -701,6 +701,112 @@ __global__ void fill_int_kernel(int *p, long long n, int v) {
   if (i < n) p[i] = v;
 }
 
+// ---- leave-one-out (Dubrule 1983) ------------------------------------------------------------------------------
+// With Q the upper-left n×n block of K⁻¹, K = [C F; Fᵀ 0], sample i left out has the residual z_i − ẑ_{−i} = w_i / Q_ii
+// and the kriging variance 1 / Q_ii, where (w, β) = K⁻¹[z; 0] are the resident dual weights. With C⁻¹ = XᵀX (X = L⁻¹,
+// lower triangular) and Y_F = X F:  Q_ii = Σ_{r>=i} X[r,i]² − W_i G_FF⁻¹ W_iᵀ,  W_i = Σ_{r>=i} X[r,i] Y_F[r,:].
+// Pass 1 reads the lower triangle of X once: CTA (column block of 64, row chunk of LOO_RCH rows) — every warp owns 8
+// columns, each a contiguous stretch of X, read by its 32 lanes in 256-byte rows, four loads in flight per lane — and
+// writes per-chunk partial sums; pass 2 reduces the chunks of a column in a fixed order (deterministic) and applies the
+// e×e algebra and the variance flags.
+constexpr int LOO_RCH = 1024;
+
+__global__ void __launch_bounds__(256) loo_colsum_kernel(const double *__restrict__ X, long long np, long long n,
+                                                         const double *__restrict__ YE, int c, long long cb0,
+                                                         double *__restrict__ partial) {
+  const long long jb = cb0 + blockIdx.x;
+  const long long r0 = jb * NB + (long long)blockIdx.y * LOO_RCH;
+  if (r0 >= n) return;
+  const long long r1 = (r0 + LOO_RCH < n) ? r0 + LOO_RCH : n;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int ns = 1 + c;
+  for (int cc = 0; cc < 8; ++cc) {
+    const long long i = jb * NB + warp * 8 + cc;
+    if (i >= n) break;
+    const double *col = X + i * np;
+    double s = 0.0, wt[GSK_MAX_DRIFT_TERMS];
+#pragma unroll
+    for (int t = 0; t < GSK_MAX_DRIFT_TERMS; ++t) wt[t] = 0.0;
+    long long r = ((r0 > i) ? r0 : i) + lane;
+    for (; r + 96 < r1; r += 128) {
+      const double x0 = col[r], x1 = col[r + 32], x2 = col[r + 64], x3 = col[r + 96];
+      s = fma(x0, x0, s); s = fma(x1, x1, s); s = fma(x2, x2, s); s = fma(x3, x3, s);
+#pragma unroll
+      for (int t = 0; t < GSK_MAX_DRIFT_TERMS; ++t)
+        if (t < c) {
+          const double *yf = YE + (long long)(1 + t) * np + r;
+          wt[t] = fma(x0, yf[0], wt[t]); wt[t] = fma(x1, yf[32], wt[t]);
+          wt[t] = fma(x2, yf[64], wt[t]); wt[t] = fma(x3, yf[96], wt[t]);
+        }
+    }
+    for (; r < r1; r += 32) {
+      const double x = col[r];
+      s = fma(x, x, s);
+#pragma unroll
+      for (int t = 0; t < GSK_MAX_DRIFT_TERMS; ++t)
+        if (t < c) wt[t] = fma(x, YE[(long long)(1 + t) * np + r], wt[t]);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+#pragma unroll
+    for (int t = 0; t < GSK_MAX_DRIFT_TERMS; ++t)
+      if (t < c)
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) wt[t] += __shfl_xor_sync(0xffffffffu, wt[t], o);
+    if (lane == 0) {
+      double *pp = partial + (long long)blockIdx.y * ns * np + i;
+      pp[0] = s;
+#pragma unroll
+      for (int t = 0; t < GSK_MAX_DRIFT_TERMS; ++t)
+        if (t < c) pp[(long long)(1 + t) * np] = wt[t];
+    }
+  }
+}
+
+__global__ void loo_epilogue_kernel(const double *__restrict__ partial, long long np, long long n, int c,
+                                    const double *__restrict__ GEE, int ne, const double *__restrict__ w,
+                                    const double4 *__restrict__ rec, long long first, long long count, unsigned flags,
+                                    GskOut out) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= count) return;
+  const long long i = first + t;
+  const int nq = (int)((n - (i / NB) * NB + LOO_RCH - 1) / LOO_RCH);
+  const int ns = 1 + c;
+  double d = 0.0, y[GSK_MAX_DRIFT_TERMS];
+  for (int j = 0; j < c; ++j) y[j] = 0.0;
+  for (int q = 0; q < nq; ++q) {
+    const double *pp = partial + (long long)q * ns * np + i;
+    d += pp[0];
+    for (int j = 0; j < c; ++j) y[j] += pp[(long long)(1 + j) * np];
+  }
+  // Q_ii = d − W G_FF⁻¹ Wᵀ = d − ‖L_F⁻¹ Wᵀ‖² with G_FF = L_F L_Fᵀ (rows/cols 1… of G_EE)
+  double Lf[GSK_MAX_DRIFT_TERMS][GSK_MAX_DRIFT_TERMS];
+  for (int j = 0; j < c; ++j) {
+    double dd = GEE[(1 + j) * ne + 1 + j];
+    for (int p = 0; p < j; ++p) dd -= Lf[j][p] * Lf[j][p];
+    dd = sqrt(dd);
+    Lf[j][j] = dd;
+    for (int a = j + 1; a < c; ++a) {
+      double s = GEE[(1 + a) * ne + 1 + j];
+      for (int p = 0; p < j; ++p) s -= Lf[a][p] * Lf[j][p];
+      Lf[a][j] = s / dd;
+    }
+  }
+  double proj = 0.0;
+  for (int j = 0; j < c; ++j) {
+    double s = y[j];
+    for (int p = 0; p < j; ++p) s -= Lf[j][p] * y[p];
+    y[j] = s / Lf[j][j];
+    proj = fma(y[j], y[j], proj);
+  }
+  const double Q = d - proj;
+  const double mu = rec[i].w - w[i] / Q;
+  double s2 = 1.0 / Q;
+  if (flags & GSK_FLAG_CLAMP_VARIANCE) s2 = (s2 > 0.0 || s2 != s2) ? s2 : 0.0;
+  if (flags & GSK_FLAG_SQRT_ROUNDTRIP) { double sd = sqrt(s2); s2 = sd * sd; }
+  gsk_store_result(out, t, mu, s2);
+}
+
 }  // namespace
 
 struct GlobalPlan {
@@ -954,6 +1060,29 @@ int gsk_global_execute(gsk_ctx *ctx, long long first, long long count, int *d_nn
   return GSK_OK;
 }
 
+int gsk_global_loo(gsk_ctx *ctx, long long first, long long count, int *d_nn, int *launches) {
+  GlobalPlan *g = ctx->gplan;
+  if (!g) { ctx->err = "global plan missing"; return GSK_ERR_STATE; }
+  cudaStream_t st = ctx->stream;
+  const long long np = g->np, n = g->n;
+  const int c = ctx->es.nterms;
+  const long long nq = (n + LOO_RCH - 1) / LOO_RCH;
+  int rc;
+  if ((rc = gsk_buf(ctx, BUF_G_PARTIAL, sizeof(double) * (size_t)nq * (1 + c) * np, (void **)&g->partial)) != GSK_OK)
+    return rc;
+  const long long cb0 = first / NB, cb1 = (first + count - 1) / NB;
+  loo_colsum_kernel<<<dim3((unsigned)(cb1 - cb0 + 1), (unsigned)nq), 256, 0, st>>>(g->X, np, n, g->YE, c, cb0, g->partial);
+  loo_epilogue_kernel<<<(unsigned)((count + 127) / 128), 128, 0, st>>>(g->partial, np, n, c, g->GEE, g->ne, g->w,
+                                                                       ctx->d_rec_orig, first, count, ctx->prob.flags,
+                                                                       ctx->out);
+  if (launches) *launches += 2;
+  if (d_nn) {
+    fill_int_kernel<<<(unsigned)((count + 255) / 256), 256, 0, st>>>(d_nn, count, (int)(n - 1));
+    if (launches) *launches += 1;
+  }
+  GSK_CUDA_CHECK(ctx, cudaGetLastError());
+  return GSK_OK;
+}
 
 // ---------------------------------------------------------------------------------------------------------------
 // LU Gaussian simulation (SURVEY §8f-4; ref src/simulation/lu.jl:75-160 preprocess, :198-224 lusim): the dense covariance

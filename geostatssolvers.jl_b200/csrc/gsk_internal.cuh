@@ -182,6 +182,7 @@ struct gsk_ctx {
   // (gsk_update_values) then skips the search — and, for explicit points, the bin sort — of the next call
   bool nbr_cached = false;
   bool nbr_reuse = false;  // armed by gsk_update_values, cleared by gsk_plan
+  bool loo = false;        // gsk_krige_loo is running: targets are the samples, each excluded from its own list
   long long nbr_first = -1, nbr_count = -1;
   int *pt_perm = nullptr;
   double *pt_sx = nullptr, *pt_sy = nullptr, *pt_sz = nullptr;
@@ -220,7 +221,8 @@ int gsk_host_stage(gsk_ctx *ctx, size_t bytes, void **out);
 int gsk_build_bins(gsk_ctx *ctx, const double *hx, const double *hy, const double *hz, const double *hv, long long n,
                    int dim, int k, bool rank_in_w = false);
 // search.cu
-int gsk_launch_search(gsk_ctx *ctx, cudaStream_t st, long long first, long long count, int *d_nn, int *d_nbr,
+// k: list length (the planned max_neighbors, or one more for leave-one-out)
+int gsk_launch_search(gsk_ctx *ctx, cudaStream_t st, long long first, long long count, int k, int *d_nn, int *d_nbr,
                       int *launches, const int *d_trank = nullptr);
 // estim.cu: the IDW / LWR per-location bodies on the neighbour lists (or on all samples when k == 0)
 int gsk_launch_simple_solver(gsk_ctx *ctx, cudaStream_t st, long long first, long long count, const int *d_nn,
@@ -233,6 +235,8 @@ int gsk_global_plan(gsk_ctx *ctx, const double *hx, const double *hy, const doub
 int gsk_global_execute(gsk_ctx *ctx, long long first, long long count, int *d_nn, int *launches);
 void gsk_global_free(gsk_ctx *ctx);
 int gsk_global_update_values(gsk_ctx *ctx);
+// leave-one-out residuals and variances of samples [first, first+count) from the resident plan (Dubrule's identities)
+int gsk_global_loo(gsk_ctx *ctx, long long first, long long count, int *d_nn, int *launches);
 int gsk_lu_plan_impl(gsk_ctx *ctx, int dim, long long nd, long long ns, const double *const *coords, const double *z1,
                      const GskVario &vg);
 int gsk_lu_sample_impl(gsk_ctx *ctx, const double *w, double *y_out);  // rec_orig carries new values: rebuild E, Y_E, G_EE (L, L⁻¹ stay)
@@ -240,6 +244,9 @@ int gsk_lu_sample_impl(gsk_ctx *ctx, const double *w, double *y_out);  // rec_or
 int gsk_points_sort(gsk_ctx *ctx, long long first, long long count, int **perm, double **sx, double **sy, double **sz);
 int gsk_points_unscatter(gsk_ctx *ctx, const int *perm, long long count, const double *ms, const double *vs,
                          const GskOut &out, const int *nn_s, int *nn_out, const int *nbr_s, int *nbr_out, int k);
+// leave-one-out: drops each sorted target's own sample index (first + perm[s]) from its (k+1)-list and cuts it to k
+int gsk_points_loo_compact(gsk_ctx *ctx, const int *perm, long long first, long long count, int k, const int *nn1,
+                           const int *nbr1, int *nn_s, int *nbr_s);
 // sgs.cu
 int gsk_sgs_plan_impl(gsk_ctx *ctx, int dim, long long n, const double *const *coords, const long long *rank,
                       const GskVario &vg, double mean, int min_neighbors, int k, double ball_radius);

@@ -84,7 +84,36 @@ __global__ void pt_unscatter_kernel(const int *__restrict__ perm, long long coun
     for (int j = 0; j < k; ++j) nbr_out[o * k + j] = nbr_s[s * k + j];
 }
 
+// Leave-one-out: sorted target s is sample first + perm[s]. Its (k+1)-list (exact (d², index) order, −1 padded beyond
+// nn1[s]) holds the k nearest samples j != i once i itself is dropped — by index, never by distance: a twin at the same
+// location stays — and the rest is cut to k. One thread per target; the k-stride lists feed the ordinary solve kernels.
+__global__ void pt_loo_compact_kernel(const int *__restrict__ perm, long long first, long long count, int k,
+                                      const int *__restrict__ nn1, const int *__restrict__ nbr1, int *__restrict__ nn_s,
+                                      int *__restrict__ nbr_s) {
+  const long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= count) return;
+  const int self = (int)(first + perm[s]);
+  const int n1 = nn1[s];
+  const int *in = nbr1 + s * (k + 1);
+  int *out = nbr_s + s * k;
+  int j = 0;
+  for (int i = 0; i < n1 && j < k; ++i) {
+    const int v = in[i];
+    if (v != self) out[j++] = v;
+  }
+  nn_s[s] = j;
+  for (int i = j; i < k; ++i) out[i] = -1;
+}
+
 }  // namespace
+
+int gsk_points_loo_compact(gsk_ctx *ctx, const int *perm, long long first, long long count, int k, const int *nn1,
+                           const int *nbr1, int *nn_s, int *nbr_s) {
+  pt_loo_compact_kernel<<<(unsigned)((count + 255) / 256), 256, 0, ctx->stream>>>(perm, first, count, k, nn1, nbr1, nn_s,
+                                                                                 nbr_s);
+  GSK_CUDA_CHECK(ctx, cudaGetLastError());
+  return GSK_OK;
+}
 
 // Sorts the points [first, first+count) by sample-lattice bin. Outputs (cached context buffers): perm[s] = slab-local
 // original index of the s-th point in sorted order, and the sorted coordinates.

@@ -588,13 +588,13 @@ __global__ void __launch_bounds__(NT, (CK && !HEAP) ? 7 : 6) search_kernel(const
 
 }  // namespace
 
-int gsk_launch_search(gsk_ctx *ctx, cudaStream_t st, long long first, long long count, int *d_nn, int *d_nbr,
+int gsk_launch_search(gsk_ctx *ctx, cudaStream_t st, long long first, long long count, int k, int *d_nn, int *d_nbr,
                       int *launches, const int *d_trank) {
   GskSearchArgs a{};
   a.trank = d_trank;
   a.tg = ctx->tg;
   a.bins = ctx->bins;
-  a.k = ctx->prob.max_neighbors;
+  a.k = k;
   a.use_ball = !(ctx->prob.ball_radius != ctx->prob.ball_radius);
   a.radius = a.use_ball ? ctx->prob.ball_radius : 0.0;
   a.first = first;

@@ -370,7 +370,7 @@ int gsk_sgs_plan_impl(gsk_ctx *ctx, int dim, long long n, const double *const *c
   const GskTargets tg_saved = ctx->tg;
   ctx->tg = tgs;
   int launches = 0;
-  rc = gsk_launch_search(ctx, st, 0, n, nn_s, nbr_s, &launches, d_trank);
+  rc = gsk_launch_search(ctx, st, 0, n, k, nn_s, nbr_s, &launches, d_trank);
   ctx->tg = tg_saved;
   if (rc != GSK_OK) return rc;
   GSK_CUDA_CHECK(ctx, cudaStreamSynchronize(st));

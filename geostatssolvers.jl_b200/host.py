@@ -19,6 +19,7 @@ into the CUDA library. There is no CPU fallback.
 """
 from __future__ import annotations
 
+import dataclasses
 import math
 import warnings
 from dataclasses import dataclass, field
@@ -600,6 +601,50 @@ def _solve_kriging(problem: EstimationProblem, solver: KrigingSolver, ctx, path_
         mus[var] = varmu
         sigmas[f"{var}_variance"] = varsigma
     return georef({**mus, **sigmas}, pdomain)                           # krig.jl:163
+
+
+def leave_one_out(data: GeoTable, solver: KrigingSolver, ctx: Optional[_abi.Context] = None) -> GeoTable:
+    """Leave-one-out cross-validation (GeoStatsValidation's ``LeaveOneOut`` folds, each solved by ``solver``) as one
+    library call per variable: row i of column `var` is sample i kriged at its own location from the other non-missing
+    samples with the same parameters, `var_variance` its kriging variance (units u and u², as `solve` gives them).
+    Every variable of the table is validated; rows whose value is missing come back masked, and so do rows with fewer
+    than `minneighbors` neighbours. Each fold holds one sample less, so `maxneighbors` is clamped to n − 1 with the
+    reference's warning. `path` does not apply (every sample is its own target)."""
+    if not isinstance(solver, KrigingSolver):
+        raise _unsupported(f"leave-one-out with {type(solver).__name__} (Kriging only)")
+    ddomain = data.domain
+    problem = EstimationProblem(data, ddomain, tuple(data.names()))
+    preproc = preprocess(problem, solver)
+    nrows = ddomain.nelements()
+    mus, sigmas = {}, {}
+    for var in problem.variables():
+        pp = dict(preproc[var])
+        samples = pp["samples"]
+        n = samples.domain.nelements()
+        if n < 2:
+            raise AssertionError(f"leave-one-out of {var} needs at least two non-missing samples")
+        local = pp["maxneighbors"] is not None
+        if local and pp["searcher"].k > n - 1:                           # the fold's own searcher_ui clamp (ui.jl:16-23)
+            warnings.warn(f"Invalid maximum number of neighbors. Adjusting to {n - 1}...")
+            pp["searcher"] = dataclasses.replace(pp["searcher"], k=n - 1)
+        spec = _problem_spec(samples, samples.domain, var, pp, local=local)
+        mean, variance, nneigh = (ctx or default_context()).krige_loo(spec, want_nneigh=True)
+        _, missing = _split_missing(uadjust(data.table[var]).values if isinstance(data.table[var], Quantities)
+                                    else data.table[var])
+        inds = np.flatnonzero(~missing)
+        mask = np.ones(nrows, dtype=bool)
+        mask[inds] = nneigh < max(int(pp["minneighbors"]), 1)
+        mu = np.full(nrows, np.nan)
+        sig = np.full(nrows, np.nan)
+        mu[inds], sig[inds] = mean, variance
+        if mask.any():
+            mu, sig = np.ma.MaskedArray(mu, mask=mask), np.ma.MaskedArray(sig, mask=mask.copy())
+        unit = pp["unit"]
+        if unit is not NoUnits:
+            mu, sig = Quantities(mu, unit), Quantities(sig, unit ** 2)
+        mus[var] = mu
+        sigmas[f"{var}_variance"] = sig
+    return georef({**mus, **sigmas}, ddomain)
 
 
 # --------------------------------------------------------------------------------------

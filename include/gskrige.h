@@ -150,7 +150,9 @@ typedef struct gsk_problem {
 
 typedef struct gsk_ctx gsk_ctx; /* opaque: one CUDA device, its stream, resident buffers */
 
-/* per-phase device times (CUDA events on the context stream) of the last gsk_execute/gsk_krige */
+/* per-phase device times (CUDA events on the context stream) of the last gsk_execute/gsk_krige/gsk_krige_loo
+ * (leave-one-out: ms_search includes the removal of each row's own index; on the global path ms_solve is the
+ * pass over L⁻¹ that yields every row's leave-one-out residual and variance) */
 typedef struct gsk_timing {
   double ms_plan;    /* H2D of samples + bin build, or global assembly + factorisation */
   double ms_search;  /* local: neighbour-search kernel(s) */
@@ -174,6 +176,16 @@ GSK_API int gsk_krige(gsk_ctx *ctx, const gsk_problem *prob,
               double *mean_out, double *var_out, /* length = slab target count */
               int32_t *nneigh_out,               /* optional: neighbours used per target (global: n_samples) */
               int32_t *neigh_idx_out);           /* optional: count × max_neighbors, 0-based, sorted by (d², idx), −1 padded */
+
+/* Leave-one-out cross-validation of the Kriging problem's samples: row i is sample i kriged from the other
+ * samples at point support (local: its k nearest j != i; global: all j != i). Targets are the samples, so
+ * grid_dims[0] = 0, n_points = 0, n_support = 1 (zero offset), target_order = NULL; target_first/target_count
+ * select a slab of SAMPLE indices (callers shard with it). solver must be GSK_SOLVER_KRIGING; n_samples >= 2;
+ * max_neighbors <= n_samples - 1 (the fold's own clamp); GSK_FLAG_REUSE_PLAN is rejected. nneigh_out /
+ * neigh_idx_out (optional, count × max_neighbors, -1 padded, never containing the row's own index) as in
+ * gsk_krige. The context holds no plan afterwards. */
+GSK_API int gsk_krige_loo(gsk_ctx *ctx, const gsk_problem *prob, double *mean_out, double *var_out,
+                          int32_t *nneigh_out, int32_t *neigh_idx_out);
 
 /* ---- single-process multi-GPU convenience (a Julia host drives all GPUs of a box from one process):
  * the slab [target_first, target_first+target_count) is split into n_devices contiguous pieces, one host

@@ -190,6 +190,61 @@ function solve_b200(problem::EstimationProblem, solver::KrigingSolver; ctx=conte
   georef((; μs..., σs...), pdomain)                                                # krig.jl:163
 end
 
+"""
+leave-one-out cross-validation of `data` with `solver` (what GeoStatsValidation's `LeaveOneOut` computes by solving one
+fold per sample): per variable one gsk_krige_loo call; row i is sample i kriged at its own location from the other
+non-missing samples. Returns `var` and `var_variance` on the data domain in data order, `missing` where the value is
+missing or fewer than `minneighbors` neighbours remain. Each fold holds n − 1 samples, so `maxneighbors` is clamped to
+n − 1 by the fold's own `searcher_ui`; `path` does not apply.
+"""
+function leaveoneout_b200(data, solver::KrigingSolver; ctx=context())
+  dtable = values(data); ddomain = domain(data)
+  μs = []; σs = []
+  for covars in covariables(EstimationProblem(data, ddomain, Tables.columnnames(Tables.columns(dtable))), solver),
+      var in covars.names
+    p = covars.params[Set([var])]
+    p.distance isa Euclidean || throw(ArgumentError("non-Euclidean `distance` is not supported by the B200 Kriging path"))
+    z = uadjust(Tables.getcolumn(Tables.columns(dtable), var))
+    inds = findall(!ismissing, z)
+    n = length(inds)
+    n >= 2 || throw(AssertionError("leave-one-out of $var needs at least two non-missing samples"))
+    sdom = view(ddomain, inds)
+    estimator = GeoStatsSolvers.kriging_ui(sdom, p.variogram, p.mean, p.degree, p.drifts)
+    islocal = !isnothing(p.maxneighbors)
+    fold = view(ddomain, inds[1:n-1])                                              # any fold: n − 1 samples
+    searcher = GeoStatsSolvers.searcher_ui(fold, p.maxneighbors, p.distance, p.neighborhood)  # the fold's clamp + warning
+    γ = estimator.γ
+    dim = embeddim(sdom)
+    X = [Float64[ustrip(coordinates(centroid(sdom, i))[d]) for i in 1:n] for d in 1:dim]
+    zs = collect(Float64, ustrip.(z[inds]))
+    est, skmean, deg = estimator isa GeoStatsModels.SimpleKriging ? (Int32(0), Float64(ustrip(estimator.μ)), Int32(0)) :
+                       estimator isa GeoStatsModels.UniversalKriging ? (Int32(2), 0.0, Int32(maximum(estimator.exponents))) :
+                       estimator isa GeoStatsModels.OrdinaryKriging ? (Int32(1), 0.0, Int32(0)) :
+                       throw(ArgumentError("ExternalDriftKriging (`drifts`) is not supported by the B200 Kriging path"))
+    k = islocal ? Int32(maxneighbors(searcher)) : Int32(0)
+    radius = (islocal && searcher isa KBallSearch) ? Float64(ustrip(Meshes.radius(searcher.ball))) : NaN
+    ptrs(v) = ntuple(d -> d <= length(v) ? pointer(v[d]) : Ptr{Float64}(C_NULL), 3)
+    μ = Vector{Float64}(undef, n); σ² = Vector{Float64}(undef, n); nn = Vector{Int32}(undef, n)
+    GC.@preserve X zs μ σ² nn begin
+      prob = GskProblem(2, dim, n, ptrs(X), pointer(zs), (0, 1, 1), (0.0, 0.0, 0.0), (1.0, 1.0, 1.0),
+        0, ntuple(_ -> Ptr{Float64}(C_NULL), 3), 0, -1, 1, ntuple(_ -> Ptr{Float64}(C_NULL), 3),
+        variokind(γ), ustrip(range(γ)), ustrip(sill(γ)), ustrip(nugget(γ)), 1e-6,
+        est, skmean, deg, Int32(p.minneighbors), k, radius, UInt32(3), Ptr{Int64}(C_NULL), Int32(0), 1.0, Int32(0))
+      check(ctx, ccall((:gsk_krige_loo, LIB), Cint,
+        (Ptr{Cvoid}, Ref{GskProblem}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}, Ptr{Int32}),
+        ctx.handle, prob, μ, σ², nn, C_NULL))
+    end
+    T = nelements(ddomain)
+    varμ = Vector{Union{Missing,Float64}}(missing, T); varσ = Vector{Union{Missing,Float64}}(missing, T)
+    ok = nn .>= max(p.minneighbors, 1)
+    varμ[inds[ok]] .= μ[ok]; varσ[inds[ok]] .= σ²[ok]
+    u = elunit(z)
+    push!(μs, var => (u == NoUnits ? varμ : varμ .* u))
+    push!(σs, Symbol(var, "_variance") => (u == NoUnits ? varσ : varσ .* u^2))
+  end
+  georef((; μs..., σs...), ddomain)
+end
+
 "drop-in for GeoStatsSolvers.solve(problem, ::IDWSolver) (idw.jl:59-148) and ::LWRSolver (lwr.jl:62-152)"
 function solve_b200(problem::EstimationProblem, solver::Union{IDWSolver,LWRSolver}; ctx=context(), devices=nothing)
   pdata = data(problem); dtable = values(pdata); ddomain = domain(pdata); pdomain = domain(problem)

@@ -17,3 +17,21 @@ sol = solve(EstimationProblem(data, grid, :z), KrigingSolver(:z => (variogram=Ga
 # compare with:  python -c "import gskrige, oracle_py; ..."  (tests/_cases.py: ref_problem_2d)
 println("known answer: mean[1:3] = ", sol.z[1:3], "  var[1:3] = ", sol.z_variance[1:3])
 println("expected from the oracle: mean[0:3] and var[0:3] of tests/_cases.ref_problem_2d(k=3)")
+
+# leave-one-out: GSKrige.leaveoneout_b200 against the reference's folds — sample i deleted, kriged at its own location
+# by KrigingSolver (what GeoStatsValidation's LeaveOneOut solves per fold). Needs libgskrige.so and a B200.
+include(joinpath(@__DIR__, "GSKrige.jl"))
+xy = [(Float64(i % 7) + 0.3 * (i % 3), Float64(i ÷ 7) + 0.2 * (i % 5)) for i in 0:48]
+loodata = georef((; z=[sin(p[1] / 2) + cos(p[2] / 3) for p in xy]), xy)
+for params in ((variogram=SphericalVariogram(range=4.0), maxneighbors=8), (variogram=ExponentialVariogram(range=5.0),))
+  solver = KrigingSolver(:z => params)
+  loo = GSKrige.leaveoneout_b200(loodata, solver)
+  worst = 0.0
+  for i in 1:length(xy)
+    keep = setdiff(1:length(xy), i)
+    fold = georef((; z=loodata.z[keep]), xy[keep])
+    ref = solve(EstimationProblem(fold, PointSet([xy[i]]), :z), solver)
+    worst = max(worst, abs(ref.z[1] - loo.z[i]), abs(ref.z_variance[1] - loo.z_variance[i]))
+  end
+  println("leave-one-out ", params, ": largest |reference fold − leaveoneout_b200| = ", worst, " (expect < 1e-9)")
+end
