@@ -267,6 +267,9 @@ def load_library(path: os.PathLike | None = None):
     lib.gsk_krige.restype = C.c_int
     lib.gsk_krige_loo.argtypes = [ctx, pp, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.gsk_krige_loo.restype = C.c_int
+    lib.gsk_krige_columns.argtypes = [ctx, pp, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_void_p]
+    lib.gsk_krige_columns.restype = C.c_int
     lib.gsk_krige_multi.argtypes = [_ip, C.c_int, pp, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_char_p, C.c_int]
     lib.gsk_krige_multi.restype = C.c_int
     lib.gsk_krige_multi_release.argtypes = []
@@ -314,7 +317,7 @@ def load_library(path: os.PathLike | None = None):
 
 
 EXPORTED_SYMBOLS = [
-    "gsk_create", "gsk_destroy", "gsk_last_error", "gsk_set_stream", "gsk_synchronize", "gsk_krige", "gsk_krige_loo", "gsk_krige_multi", "gsk_krige_multi_release", "gsk_plan",
+    "gsk_create", "gsk_destroy", "gsk_last_error", "gsk_set_stream", "gsk_synchronize", "gsk_krige", "gsk_krige_loo", "gsk_krige_columns", "gsk_krige_multi", "gsk_krige_multi_release", "gsk_plan",
     "gsk_execute", "gsk_execute_peers", "gsk_update_values", "gsk_lu_plan", "gsk_lu_sample", "gsk_sgs_plan", "gsk_sgs_sample", "gsk_sgs_sample_device", "gsk_sgs_weights", "gsk_get_timing", "gsk_set_phase_timing", "gsk_num_targets", "gsk_uk_exponents", "gsk_default_support",
     "gsk_measure_fp64_peak", "gsk_abi_version",
 ]
@@ -396,6 +399,44 @@ class Context:
         if want_nneigh:
             return mean, var, nneigh
         return mean, var
+
+    def krige_columns(self, spec: ProblemSpec, Z, want_nneigh: bool = False, want_neighbors: bool = False,
+                      want_weights: bool = False):
+        """Kriging of every column of ``Z`` (n_samples × m) over the spec's samples in one call (``gsk_krige_columns``):
+        the search and the factorisations run once. The spec's own values are not used. Returns ``mean`` (count × m)
+        and ``var`` (count), then — as requested — the neighbour counts, the count × k neighbour lists, and the
+        count × k Kriging weights with the count × nterms Lagrange multipliers (local path only)."""
+        Z = np.ascontiguousarray(Z, dtype=np.float64)
+        if Z.ndim != 2 or Z.shape[0] != spec.n_samples or Z.shape[1] < 1:
+            raise ValueError(f"Z must have shape (n_samples, m >= 1) = ({spec.n_samples}, m), got {Z.shape}")
+        first, count = spec.slab
+        m = Z.shape[1]
+        k = spec.params["max_neighbors"]
+        if want_weights and k == 0:
+            raise ValueError("weights are returned by the local path only (max_neighbors > 0)")
+        nterms = {EST_SIMPLE: 0, EST_ORDINARY: 1}.get(spec.params["estimator"])
+        if nterms is None:
+            nterms = len(uk_exponents(spec.params["uk_degree"], spec.dim))
+        mean = np.empty((count, m), dtype=np.float64)
+        var = np.empty(count, dtype=np.float64)
+        nneigh = np.empty(count, dtype=np.int32) if (want_neighbors or want_nneigh) else None
+        idx = np.empty((count, max(k, 1)), dtype=np.int32) if (want_neighbors and k > 0) else None
+        w = np.empty((count, k), dtype=np.float64) if want_weights else None
+        lag = np.empty((count, nterms), dtype=np.float64) if (want_weights and nterms > 0) else None
+        ps = spec.c_struct()
+        ps.values = None
+        ptr = lambda a: a.ctypes.data if a is not None else None  # noqa: E731
+        rc = self.lib.gsk_krige_columns(self._h, C.byref(ps), m, Z.ctypes.data, mean.ctypes.data, var.ctypes.data,
+                                        ptr(nneigh), ptr(idx), ptr(w), ptr(lag))
+        self._check(rc)
+        out = [mean, var]
+        if want_nneigh or want_neighbors:
+            out.append(nneigh)
+        if want_neighbors:
+            out.append(idx)
+        if want_weights:
+            out += [w, lag if lag is not None else np.empty((count, 0))]
+        return tuple(out)
 
     def krige_into(self, spec: ProblemSpec, mean: np.ndarray, var: np.ndarray):
         """Same as :meth:`krige` but writes into caller-provided (e.g. pinned) host arrays."""

@@ -614,7 +614,9 @@ static int execute_impl(gsk_ctx *ctx, int64_t first, int64_t count, int32_t *d_n
       rc = gsk_launch_search(ctx, ctx->stream, 0, count, k, nn_s, nbr_s, &launches);
     }
     if (phase_timing) cudaEventRecord(ctx->ev[4], ctx->stream);
+    ctx->cols.perm = perm;  // the columns epilogue writes its rows in slab order itself
     if (rc == GSK_OK) rc = launch_body(ctx->stream, 0, count, nn_s, nbr_s, 0);
+    ctx->cols.perm = nullptr;
     ctx->tg = tg_saved;
     ctx->out = out_saved;
     if (rc != GSK_OK) return rc;
@@ -1053,6 +1055,90 @@ extern "C" GSK_API int gsk_krige_loo(gsk_ctx *ctx, const gsk_problem *p, double 
 } catch (const std::exception &e) {
   if (ctx) { ctx->loo = false; cudaStreamSynchronize(ctx->stream2); cudaStreamSynchronize(ctx->stream); free_plan(ctx); }
   return fail(ctx, GSK_ERR_STATE, std::string("gsk_krige_loo: ") + e.what());
+}
+
+// ---------------------------------------------------------------------------------------------
+// many value columns over one sample set: the geometry (search, factorisation) once, applied to every column
+// ---------------------------------------------------------------------------------------------
+extern "C" GSK_API int gsk_krige_columns(gsk_ctx *ctx, const gsk_problem *p, int32_t n_cols, const double *values,
+                                         double *mean_out, double *var_out, int32_t *nneigh_out, int32_t *neigh_idx_out,
+                                         double *weights_out, double *lagrange_out) try {
+  if (!ctx) return GSK_ERR_INVALID;
+  if (!mean_out || !var_out) return fail(ctx, GSK_ERR_INVALID, "mean_out / var_out are NULL");
+  if (!p) return fail(ctx, GSK_ERR_INVALID, "problem is NULL");
+  if (p->values)
+    return fail(ctx, GSK_ERR_INVALID, "gsk_krige_columns: prob->values must be NULL (the values are the columns)");
+  if (n_cols < 1 || !values) return fail(ctx, GSK_ERR_INVALID, "gsk_krige_columns: n_cols must be >= 1 and values non-NULL");
+  if (p->flags & GSK_FLAG_REUSE_PLAN)
+    return fail(ctx, GSK_ERR_INVALID, "gsk_krige_columns: GSK_FLAG_REUSE_PLAN does not apply (no plan is kept)");
+  if (p->solver != GSK_SOLVER_KRIGING)
+    return fail(ctx, GSK_ERR_UNSUPPORTED, "gsk_krige_columns: implemented for the Kriging solver only");
+  if (p->max_neighbors == 0 && (weights_out || lagrange_out))
+    return fail(ctx, GSK_ERR_INVALID, "gsk_krige_columns: weights_out / lagrange_out are for the local path only "
+                                      "(max_neighbors > 0)");
+  if (p->n_samples < 1) return fail(ctx, GSK_ERR_INVALID, "n_samples must be >= 1");
+  const long long n = p->n_samples;
+  const int m = n_cols;
+  // the plan takes column 0 as its values (the kernels' own single-column mean is computed and discarded)
+  std::vector<double> v0((size_t)n);
+  for (long long i = 0; i < n; ++i) v0[(size_t)i] = values[(size_t)i * m];
+  gsk_problem q = *p;
+  q.values = v0.data();
+  int rc = gsk_plan(ctx, &q);
+  const int64_t first = p->target_first, count = rc == GSK_OK ? (p->target_count < 0 ? ctx->n_targets - first : p->target_count) : 0;
+  const int k = p->max_neighbors, c = ctx->nterms;
+  // pieces of the slab whose per-column means fit in 2 GiB of device memory
+  const long long piece = std::max<long long>(1, std::min<long long>(count, (2ll << 30) / (8ll * m)));
+  double *d_z = nullptr, *d_cm = nullptr, *d_mv = nullptr, *d_w = nullptr, *d_lag = nullptr;
+  auto copy_out = [&](void *dst, const void *src, size_t bytes) -> int {
+    GSK_CUDA_CHECK(ctx, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    return GSK_OK;
+  };
+  if (rc == GSK_OK && count > 0) rc = gsk_buf(ctx, BUF_C_Z, sizeof(double) * (size_t)n * m, (void **)&d_z);
+  if (rc == GSK_OK && count > 0) rc = gsk_buf(ctx, BUF_C_MEAN, sizeof(double) * (size_t)piece * m, (void **)&d_cm);
+  if (rc == GSK_OK && count > 0) rc = gsk_buf(ctx, BUF_C_MV, sizeof(double) * 2 * (size_t)piece, (void **)&d_mv);
+  if (rc == GSK_OK && count > 0 && weights_out) rc = gsk_buf(ctx, BUF_C_W, sizeof(double) * (size_t)piece * k, (void **)&d_w);
+  if (rc == GSK_OK && count > 0 && lagrange_out && c > 0)
+    rc = gsk_buf(ctx, BUF_C_LAG, sizeof(double) * (size_t)piece * c, (void **)&d_lag);
+  if (rc == GSK_OK && count > 0 && nneigh_out) rc = ensure(ctx, (void **)&ctx->d_nn_out, &ctx->cap_nn_out, sizeof(int) * (size_t)piece);
+  if (rc == GSK_OK && count > 0 && neigh_idx_out && k > 0)
+    rc = ensure(ctx, (void **)&ctx->d_nbr_out, &ctx->cap_nbr_out, sizeof(int) * (size_t)piece * k);
+  if (rc == GSK_OK && count > 0) {
+    if (cudaMemcpyAsync(d_z, values, sizeof(double) * (size_t)n * m, cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess)
+      rc = fail(ctx, GSK_ERR_CUDA, "gsk_krige_columns: value upload failed");
+    ctx->cols = GskCols{};
+    ctx->cols.active = true;
+    ctx->cols.z = d_z;
+    ctx->cols.m = m;
+    ctx->cols.mean = d_cm;
+    ctx->cols.w = d_w;
+    ctx->cols.lag = d_lag;
+    if (rc == GSK_OK && k == 0) rc = gsk_global_column_weights(ctx, d_z, m);
+    for (long long off = 0; off < count && rc == GSK_OK; off += piece) {
+      const long long cnt = std::min<long long>(piece, count - off);
+      int *d_nn = nneigh_out ? ctx->d_nn_out : nullptr, *d_idx = (neigh_idx_out && k > 0) ? ctx->d_nbr_out : nullptr;
+      rc = gsk_execute(ctx, first + off, cnt, d_mv, d_mv + piece, d_nn, d_idx);
+      if (rc == GSK_OK) rc = copy_out(mean_out + off * m, d_cm, sizeof(double) * (size_t)cnt * m);
+      if (rc == GSK_OK) rc = copy_out(var_out + off, d_mv + piece, sizeof(double) * (size_t)cnt);
+      if (rc == GSK_OK && d_nn) rc = copy_out(nneigh_out + off, d_nn, sizeof(int) * (size_t)cnt);
+      if (rc == GSK_OK && d_idx) rc = copy_out(neigh_idx_out + off * k, d_idx, sizeof(int) * (size_t)cnt * k);
+      if (rc == GSK_OK && d_w) rc = copy_out(weights_out + off * k, d_w, sizeof(double) * (size_t)cnt * k);
+      if (rc == GSK_OK && d_lag) rc = copy_out(lagrange_out + off * c, d_lag, sizeof(double) * (size_t)cnt * c);
+      if (rc == GSK_OK) GSK_CUDA_CHECK(ctx, cudaStreamSynchronize(ctx->stream));  // the next piece reuses the buffers
+    }
+    ctx->timing.targets = count;
+  }
+  // like gsk_krige_loo: nothing of this call's plan serves a later gsk_execute
+  cudaStreamSynchronize(ctx->stream);
+  ctx->cols = GskCols{};
+  free_plan(ctx);
+  return rc;
+} catch (const std::bad_alloc &) {  // no exception may cross the C ABI
+  if (ctx) { cudaStreamSynchronize(ctx->stream); ctx->cols = GskCols{}; free_plan(ctx); }
+  return fail(ctx, GSK_ERR_NOMEM, "gsk_krige_columns: out of host memory");
+} catch (const std::exception &e) {
+  if (ctx) { cudaStreamSynchronize(ctx->stream); ctx->cols = GskCols{}; free_plan(ctx); }
+  return fail(ctx, GSK_ERR_STATE, std::string("gsk_krige_columns: ") + e.what());
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -807,6 +807,70 @@ __global__ void loo_epilogue_kernel(const double *__restrict__ partial, long lon
   gsk_store_result(out, t, mu, s2);
 }
 
+// ---- gsk_krige_columns ---------------------------------------------------------------------------------------
+// E's value column from column j of the n × m sample-major values (− μ for Simple Kriging); padded rows stay 0
+__global__ void set_e_column_kernel(const double *__restrict__ Z, int m, int j, long long n, double shift,
+                                    double *__restrict__ E) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) E[i] = Z[(size_t)i * m + j] - shift;
+}
+
+// Per-column means of a target batch from the dual weights: mean[t, j] = Σ_i B[i, t]·W[i, j] + β_j·f₀(t) (+ μ for
+// Simple Kriging) — the same dual form as the single-column mean (dual_mean_kernel + global_epilogue_kernel), as one
+// GEMM Bᵀ W on the FP64 tensor path. One warp per 16 targets × 8 columns, mma.m16n8k16 over the padded sample axis
+// (np is a multiple of 16; the batch's padded target columns of B and the padded columns of W are zero). Every output
+// element sees only its own row of Bᵀ and column of W, in the same k order, so a column's result does not depend on
+// m or on its position.
+__global__ void __launch_bounds__(128) cols_mean_kernel(const double *__restrict__ Bm, long long np, int nb,
+                                                        const double *__restrict__ W, int m, int m8,
+                                                        const double *__restrict__ beta, GskEstimator es, GskTargets tg,
+                                                        long long first, double *__restrict__ out) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t4 = lane & 3;
+  const long long t0 = (long long)blockIdx.x * 16;
+  const int j0 = (blockIdx.y * 4 + warp) * 8;
+  if (j0 >= m8) return;
+  const double *a0 = Bm + (t0 + g) * np + t4, *a1 = a0 + 8 * np;
+  const double *b0 = W + (long long)(j0 + g) * np + t4;
+  double d[4] = {0.0, 0.0, 0.0, 0.0};
+  for (long long k0 = 0; k0 < np; k0 += 16) {
+    const double af[8] = {a0[k0], a1[k0], a0[k0 + 4], a1[k0 + 4], a0[k0 + 8], a1[k0 + 8], a0[k0 + 12], a1[k0 + 12]};
+    const double bf[4] = {b0[k0], b0[k0 + 4], b0[k0 + 8], b0[k0 + 12]};
+    asm volatile(
+        "mma.sync.aligned.m16n8k16.row.col.f64.f64.f64.f64 {%0,%1,%2,%3}, {%4,%5,%6,%7,%8,%9,%10,%11}, "
+        "{%12,%13,%14,%15}, {%0,%1,%2,%3};"
+        : "+d"(d[0]), "+d"(d[1]), "+d"(d[2]), "+d"(d[3])
+        : "d"(af[0]), "d"(af[1]), "d"(af[2]), "d"(af[3]), "d"(af[4]), "d"(af[5]), "d"(af[6]), "d"(af[7]), "d"(bf[0]),
+          "d"(bf[1]), "d"(bf[2]), "d"(bf[3]));
+  }
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    const long long t = t0 + g + 8 * h;
+    if (t >= nb) continue;
+    double f0[GSK_MAX_DRIFT_TERMS];
+    if (es.nterms > 0) {
+      double tc[3];
+      gsk_target_center(tg, first + t, tc);
+      for (int q = 0; q < es.nterms; ++q)
+        f0[q] = (es.kind == GSK_EST_ORDINARY)
+                    ? 1.0
+                    : gsk_ipow(tc[0], es.exps[q][0]) * gsk_ipow(tc[1], es.exps[q][1]) * gsk_ipow(tc[2], es.exps[q][2]);
+    }
+#pragma unroll
+    for (int cc = 0; cc < 2; ++cc) {
+      const int j = j0 + 2 * t4 + cc;
+      if (j >= m) continue;
+      double mu = d[2 * h + cc];
+      if (es.kind == GSK_EST_SIMPLE) mu = es.sk_mean + mu;
+      else {
+        double mb = 0.0;
+        for (int q = 0; q < es.nterms; ++q) mb += beta[j * GSK_MAX_DRIFT_TERMS + q] * f0[q];
+        mu = mu + mb;
+      }
+      out[t * m + j] = mu;
+    }
+  }
+}
+
 }  // namespace
 
 struct GlobalPlan {
@@ -1005,6 +1069,37 @@ int gsk_global_update_values(gsk_ctx *ctx) {
   return global_dual_weights(ctx);
 }
 
+int gsk_global_column_weights(gsk_ctx *ctx, const double *d_z, int m) {
+  GlobalPlan *g = ctx->gplan;
+  if (!g) { ctx->err = "global plan missing"; return GSK_ERR_STATE; }
+  cudaStream_t st = ctx->stream;
+  const long long np = g->np;
+  const double shift = (ctx->es.kind == GSK_EST_SIMPLE) ? ctx->es.sk_mean : 0.0;
+  const int m8 = (m + 7) / 8 * 8;
+  int rc;
+  if ((rc = gsk_buf(ctx, BUF_C_GW, sizeof(double) * (size_t)np * m8, (void **)&ctx->cols.gw)) != GSK_OK) return rc;
+  if ((rc = gsk_buf(ctx, BUF_C_GBETA, sizeof(double) * (size_t)m * GSK_MAX_DRIFT_TERMS, (void **)&ctx->cols.gbeta)) != GSK_OK)
+    return rc;
+  if (m8 > m)  // padding columns of the column-mean GEMM
+    GSK_CUDA_CHECK(ctx, cudaMemsetAsync(ctx->cols.gw + (size_t)m * np, 0, sizeof(double) * (size_t)(m8 - m) * np, st));
+  std::vector<double> hbeta((size_t)m * GSK_MAX_DRIFT_TERMS);
+  // column by column through the plan's own refinement (gsk_global_update_values without the record upload): only
+  // E's value column, its row of Y_E and of G_EE change
+  for (int j = 0; j < m; ++j) {
+    set_e_column_kernel<<<(unsigned)((g->n + 255) / 256), 256, 0, st>>>(d_z, m, j, g->n, shift, g->E);
+    linv_times_e_kernel<<<(unsigned)((np + 7) / 8), 256, 0, st>>>(g->X, np, np, g->E, 1, g->YE);
+    gram_ee_kernel<<<1, 256, 0, st>>>(g->YE, np, g->ne, g->GEE);
+    GSK_CUDA_CHECK(ctx, cudaGetLastError());
+    if ((rc = global_dual_weights(ctx)) != GSK_OK) return rc;
+    GSK_CUDA_CHECK(ctx, cudaMemcpyAsync(ctx->cols.gw + (size_t)j * np, g->w, sizeof(double) * (size_t)np,
+                                        cudaMemcpyDeviceToDevice, st));
+    for (int q = 0; q < GSK_MAX_DRIFT_TERMS; ++q) hbeta[(size_t)j * GSK_MAX_DRIFT_TERMS + q] = g->beta[q];
+  }
+  GSK_CUDA_CHECK(ctx, cudaMemcpyAsync(ctx->cols.gbeta, hbeta.data(), sizeof(double) * hbeta.size(), cudaMemcpyHostToDevice, st));
+  GSK_CUDA_CHECK(ctx, cudaStreamSynchronize(st));  // hbeta leaves scope
+  return GSK_OK;
+}
+
 int gsk_global_execute(gsk_ctx *ctx, long long first, long long count, int *d_nn, int *launches) {
   GlobalPlan *g = ctx->gplan;
   if (!g) { ctx->err = "global plan missing"; return GSK_ERR_STATE; }
@@ -1051,6 +1146,12 @@ int gsk_global_execute(gsk_ctx *ctx, long long first, long long count, int *d_nn
                                                              ctx->tg, ctx->vg.sill, ctx->prob.flags, first + off,
                                                              out_b, dual);
     if (launches) *launches += 4;
+    if (ctx->cols.active) {
+      const int m = ctx->cols.m, m8 = (m + 7) / 8 * 8;
+      cols_mean_kernel<<<dim3((unsigned)((nb + 15) / 16), (unsigned)((m8 / 8 + 3) / 4)), 128, 0, st>>>(
+          g->Bm, np, nb, ctx->cols.gw, m, m8, ctx->cols.gbeta, ctx->es, ctx->tg, first + off, ctx->cols.mean + off * m);
+      if (launches) *launches += 1;
+    }
   }
   if (d_nn) {
     fill_int_kernel<<<(unsigned)((count + 255) / 256), 256, 0, st>>>(d_nn, count, (int)g->n);

@@ -101,6 +101,31 @@ struct GskLocalArgs {
   GskOut out;               // outputs, indexed by slab-local target (pointers already offset)
 };
 
+// gsk_krige_columns: what the column-packed kernel's columns epilogue reads (a kernel parameter of its own, after the
+// others, so that GskLocalArgs and the code of every other kernel stay as they are). Row r of every output is
+// slab-local target r (cperm, when set, maps a bin-sorted target to its row); pointers already offset.
+struct GskColArgs {
+  const double *z;  // n_samples × ncols values, sample-major
+  int ncols;
+  const int *perm;
+  double *mean;     // count × ncols
+  double *w;        // optional: count × k Kriging weights
+  double *lag;      // optional: count × nterms Lagrange multipliers
+};
+
+// state of a running gsk_krige_columns (device pointers; row 0 of each output is the first target of the call)
+struct GskCols {
+  bool active = false;
+  const double *z = nullptr;  // n_samples × m
+  int m = 0;
+  double *mean = nullptr;     // count × m
+  double *w = nullptr;        // local path, optional: count × k
+  double *lag = nullptr;      // local path, optional: count × nterms
+  const int *perm = nullptr;  // explicit points: bin-sorted target → slab-local row (set inside gsk_execute)
+  double *gw = nullptr;       // global path: refined dual weights, np × m8 (m8 = m rounded up to 8, zero columns)
+  double *gbeta = nullptr;    // global path: their drift coefficients, m × GSK_MAX_DRIFT_TERMS
+};
+
 struct GskSearchArgs {
   GskTargets tg;
   GskBins bins;
@@ -135,7 +160,8 @@ struct SgsPlan;     // sgs.cu
 enum GskBufId {
   BUF_REC_ORIG, BUF_REC_SORTED, BUF_CELL_START, BUF_SUP, BUF_PTS0, BUF_PTS1, BUF_PTS2, BUF_CELL_OF, BUF_COUNTS,
   BUF_G_A, BUF_G_X, BUF_G_DINV, BUF_G_E, BUF_G_YE, BUF_G_GEE, BUF_G_BM, BUF_G_PARTIAL, BUF_G_W, BUF_G_TMP, BUF_G_DMEAN, BUF_PEAK,
-  BUF_PT_CELL, BUF_PT_COUNTS, BUF_PT_PERM, BUF_PT_X, BUF_PT_Y, BUF_PT_Z, BUF_PT_MEAN, BUF_PT_VAR, BUF_PT_NN, BUF_PT_NBR, BUF_VALS, BUF_REDO, BUF_COUNT
+  BUF_PT_CELL, BUF_PT_COUNTS, BUF_PT_PERM, BUF_PT_X, BUF_PT_Y, BUF_PT_Z, BUF_PT_MEAN, BUF_PT_VAR, BUF_PT_NN, BUF_PT_NBR, BUF_VALS, BUF_REDO,
+  BUF_C_Z, BUF_C_MEAN, BUF_C_MV, BUF_C_W, BUF_C_LAG, BUF_C_GW, BUF_C_GBETA, BUF_COUNT
 };
 
 struct gsk_ctx {
@@ -183,6 +209,7 @@ struct gsk_ctx {
   bool nbr_cached = false;
   bool nbr_reuse = false;  // armed by gsk_update_values, cleared by gsk_plan
   bool loo = false;        // gsk_krige_loo is running: targets are the samples, each excluded from its own list
+  GskCols cols;            // gsk_krige_columns is running: the solve also writes per-column means (and weights)
   long long nbr_first = -1, nbr_count = -1;
   int *pt_perm = nullptr;
   double *pt_sx = nullptr, *pt_sy = nullptr, *pt_sz = nullptr;
@@ -237,6 +264,9 @@ void gsk_global_free(gsk_ctx *ctx);
 int gsk_global_update_values(gsk_ctx *ctx);
 // leave-one-out residuals and variances of samples [first, first+count) from the resident plan (Dubrule's identities)
 int gsk_global_loo(gsk_ctx *ctx, long long first, long long count, int *d_nn, int *launches);
+// gsk_krige_columns: refined dual weights (w, β) of each of the m value columns d_z (n × m, sample-major) into
+// ctx->cols.gw / gbeta, each exactly as a plan with that column as its values computes them
+int gsk_global_column_weights(gsk_ctx *ctx, const double *d_z, int m);
 int gsk_lu_plan_impl(gsk_ctx *ctx, int dim, long long nd, long long ns, const double *const *coords, const double *z1,
                      const GskVario &vg);
 int gsk_lu_sample_impl(gsk_ctx *ctx, const double *w, double *y_out);  // rec_orig carries new values: rebuild E, Y_E, G_EE (L, L⁻¹ stay)

@@ -351,9 +351,10 @@ __device__ __forceinline__ void rhs_tensor3(const GskLocalArgs &a, const GskVari
 }
 
 // G lanes per target, R register row slots (R·G >= RS), W panel width, RS rows stored per column,
-// NT threads per CTA
-template <int G, int R, int W, int RS, int NT, int DIM, int VK>
-__global__ void __launch_bounds__(NT) local_solve_kernel(const GskLocalArgs a, const Layout L) {
+// NT threads per CTA. COLS: the gsk_krige_columns epilogue (Kriging weights, then one mean per value column) follows
+// phase 6; the instantiations without it compile to the same code as before it existed.
+template <int G, int R, int W, int RS, int NT, int DIM, int VK, bool COLS = false>
+__global__ void __launch_bounds__(NT) local_solve_kernel(const GskLocalArgs a, const Layout L, const GskColArgs ca) {
   static_assert(R * G >= RS && RS % W == 0, "register rows must cover the stored rows");
   constexpr int CTA_THREADS = NT;
   constexpr int RT = RS;
@@ -846,6 +847,7 @@ __global__ void __launch_bounds__(NT) local_solve_kernel(const GskLocalArgs a, c
         const double nu = (gfb - f0) / gff;
         mean = gbz - gfz * nu;
         var = vg.sill - (gbb - gfb * nu + f0 * nu);
+        if constexpr (COLS) GM[EPr] = nu;  // row 1 (the z row) is free: the columns epilogue reads ν from there
       } else {
         // solve Gff ν = gfb − f0 (c×c SPD) by Cholesky in place on GM
         double f0[GSK_MAX_DRIFT_TERMS], nu[GSK_MAX_DRIFT_TERMS];
@@ -888,11 +890,70 @@ __global__ void __launch_bounds__(NT) local_solve_kernel(const GskLocalArgs a, c
         }
         mean = gbz - mz;
         var = vg.sill - (gbb - mb + mf);
+        if constexpr (COLS)
+          for (int j = 0; j < c; ++j) GM[EPr + j] = nu[j];
       }
       if (a.flags & GSK_FLAG_CLAMP_VARIANCE) var = (var > 0.0 || var != var) ? var : 0.0;
       if (a.flags & GSK_FLAG_SQRT_ROUNDTRIP) { double sd = sqrt(var); var = sd * sd; }
     }
     gsk_store_result(a.out, t, mean, var);
+  }
+
+  // ---- columns epilogue (gsk_krige_columns): λ from Lᵀλ = y_b − Y_F ν, then mean_j = Σ λ_i z[nbr_i, j] ----
+  if constexpr (COLS) {
+    __syncwarp();
+    const int c = a.es.nterms;
+    // lane l keeps w_i for rows i = l + G·s (column i of the packed factor starts at cb[s]); the extra rows of column
+    // i hold y_b (row KC) and y_F (rows KC + 2 …). Rows past nn are identity with zero extra entries: w_i = λ_i = 0.
+    double wv[JM];
+    int cb[JM];
+#pragma unroll
+    for (int s = 0; s < JM; ++s) {
+      const int i = s * G + l;
+      cb[s] = col_off<LD, A>(i) - (i & ~(A - 1));
+      double v = 0.0;
+      if (i < KC && estimate) {
+        v = S[cb[s] + KC];
+        for (int q = 0; q < c; ++q) v = fma(-GM[EPr + q], S[cb[s] + KC + 2 + q], v);
+      }
+      wv[s] = v;
+    }
+    // backward substitution, column form: λ_j = w_j / L_jj is final, then w_i −= L[j][i]·λ_j for i < j (L[j][i] is
+    // row j of packed column i). λ goes to nbX, free since phase 3.
+    for (int j = KC - 1; j >= 0; --j) {
+      const int sj = j / G, lj = j - sj * G;
+      double wj = 0.0;
+#pragma unroll
+      for (int s = 0; s < JM; ++s) wj = (s == sj) ? wv[s] : wj;
+      wj = __shfl_sync(0xffffffffu, wj, gbase + lj);
+      const double lam = wj / S[col_off<LD, A>(j) - (j & ~(A - 1)) + j];
+      if (l == lj) nbX[j] = lam;
+#pragma unroll
+      for (int s = 0; s < JM; ++s) {
+        const int i = s * G + l;
+        if (i < j) wv[s] = fma(-S[cb[s] + j], lam, wv[s]);
+      }
+    }
+    int *nbi = reinterpret_cast<int *>(nbY);  // neighbour indices next to λ (nbY holds KCMAX doubles)
+    for (int i = l; i < nn; i += G) nbi[i] = a.nbr[t * a.k + i];
+    __syncwarp();
+    if (live) {
+      const long long row = ca.perm ? (long long)ca.perm[t] : t;
+      const int m = ca.ncols;
+      const bool sk = a.es.kind == GSK_EST_SIMPLE;
+      const double mu = sk ? a.es.sk_mean : 0.0;
+      // one column per lane: a neighbour's m values are contiguous, the lanes of a group read them together; the sum
+      // runs over i in list order whatever the configuration, so a column's mean does not depend on m or its position
+      for (int col = l; col < m; col += G) {
+        double acc = 0.0;
+        for (int i = 0; i < nn; ++i) acc = fma(nbX[i], ca.z[(size_t)nbi[i] * m + col] - mu, acc);
+        ca.mean[row * m + col] = estimate ? mu + acc : NAN;
+      }
+      if (ca.w)
+        for (int i = l; i < a.k; i += G) ca.w[row * a.k + i] = (estimate && i < nn) ? nbX[i] : 0.0;
+      if (ca.lag)
+        for (int q = l; q < c; q += G) ca.lag[row * c + q] = estimate ? GM[EPr + q] : NAN;
+    }
   }
 #undef GSK_ROW_OK
 #undef ROW0
@@ -900,8 +961,8 @@ __global__ void __launch_bounds__(NT) local_solve_kernel(const GskLocalArgs a, c
 #undef OWNER_SLOT
 }
 
-template <int G, int R, int W, int RS, int NT, int DIM, int VK>
-inline cudaError_t launch_one(const GskLocalArgs &a, int e, cudaStream_t st) {
+template <int G, int R, int W, int RS, int NT, int DIM, int VK, bool COLS>
+inline cudaError_t launch_one(const GskLocalArgs &a, const GskColArgs &ca, int e, cudaStream_t st) {
   constexpr int CTA_THREADS = NT;
   constexpr int TPW = 32 / G;
   constexpr int TPC = TPW * (CTA_THREADS / 32);
@@ -916,32 +977,32 @@ inline cudaError_t launch_one(const GskLocalArgs &a, int e, cudaStream_t st) {
   b.sup_smem = (a.nsup <= GSK_MAX_SUPPORT && smem <= GSK_SMEM_OPTIN_MAX) ? 1 : 0;
   if (!b.sup_smem) smem = sizeof(double) * ((size_t)CTAB + (size_t)TPC * L.gsz);
   if (smem > GSK_SMEM_OPTIN_MAX) return cudaErrorInvalidConfiguration;  // reported as GSK_ERR_UNSUPPORTED by the caller
-  auto kern = local_solve_kernel<G, R, W, RS, NT, DIM, VK>;
+  auto kern = local_solve_kernel<G, R, W, RS, NT, DIM, VK, COLS>;
   cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (err != cudaSuccess) return err;
   unsigned grid = (unsigned)((a.count + TPC - 1) / TPC);
-  kern<<<grid, CTA_THREADS, smem, st>>>(b, L);
+  kern<<<grid, CTA_THREADS, smem, st>>>(b, L, ca);
   return cudaGetLastError();
 }
 
-template <int G, int R, int W, int RS, int NT>
-inline cudaError_t launch_cfg(const GskLocalArgs &a, int e, cudaStream_t st) {
+template <int G, int R, int W, int RS, int NT, bool COLS = false>
+inline cudaError_t launch_cfg(const GskLocalArgs &a, const GskColArgs &ca, int e, cudaStream_t st) {
   const bool d3 = a.tg.dim == 3;
   switch (a.vg.kind) {
     case GSK_VARIO_GAUSSIAN:
-      return d3 ? launch_one<G, R, W, RS, NT, 3, GSK_VARIO_GAUSSIAN>(a, e, st) : launch_one<G, R, W, RS, NT, 2, GSK_VARIO_GAUSSIAN>(a, e, st);
+      return d3 ? launch_one<G, R, W, RS, NT, 3, GSK_VARIO_GAUSSIAN, COLS>(a, ca, e, st) : launch_one<G, R, W, RS, NT, 2, GSK_VARIO_GAUSSIAN, COLS>(a, ca, e, st);
     case GSK_VARIO_SPHERICAL:
-      return d3 ? launch_one<G, R, W, RS, NT, 3, GSK_VARIO_SPHERICAL>(a, e, st) : launch_one<G, R, W, RS, NT, 2, GSK_VARIO_SPHERICAL>(a, e, st);
+      return d3 ? launch_one<G, R, W, RS, NT, 3, GSK_VARIO_SPHERICAL, COLS>(a, ca, e, st) : launch_one<G, R, W, RS, NT, 2, GSK_VARIO_SPHERICAL, COLS>(a, ca, e, st);
     default:
-      return d3 ? launch_one<G, R, W, RS, NT, 3, GSK_VARIO_EXPONENTIAL>(a, e, st) : launch_one<G, R, W, RS, NT, 2, GSK_VARIO_EXPONENTIAL>(a, e, st);
+      return d3 ? launch_one<G, R, W, RS, NT, 3, GSK_VARIO_EXPONENTIAL, COLS>(a, ca, e, st) : launch_one<G, R, W, RS, NT, 2, GSK_VARIO_EXPONENTIAL, COLS>(a, ca, e, st);
   }
 }
 
 }  // namespace gsk_local
 
-// one translation unit per register/lanes configuration (compiled in parallel)
-cudaError_t gsk_local_launch_A(const GskLocalArgs &a, int e, cudaStream_t st);  // G=4  R=3 W=4  12 rows, 128 thr
-cudaError_t gsk_local_launch_B(const GskLocalArgs &a, int e, cudaStream_t st);  // G=4  R=6 W=4  24 rows, 128 thr
-cudaError_t gsk_local_launch_C(const GskLocalArgs &a, int e, cudaStream_t st);  // G=8  R=5 W=8  40 rows,  64 thr
-cudaError_t gsk_local_launch_D(const GskLocalArgs &a, int e, cudaStream_t st);  // G=32 R=3 W=8  72 rows, 128 thr
-cudaError_t gsk_local_launch_E(const GskLocalArgs &a, int e, cudaStream_t st);  // G=32 R=4 W=8 112 rows, 128 thr
+// one translation unit per register/lanes configuration (compiled in parallel); cols: run the gsk_krige_columns epilogue
+cudaError_t gsk_local_launch_A(const GskLocalArgs &a, int e, cudaStream_t st, const GskColArgs *cols = nullptr);  // G=4  R=3 W=4  12 rows, 128 thr
+cudaError_t gsk_local_launch_B(const GskLocalArgs &a, int e, cudaStream_t st, const GskColArgs *cols = nullptr);  // G=4  R=6 W=4  24 rows, 128 thr
+cudaError_t gsk_local_launch_C(const GskLocalArgs &a, int e, cudaStream_t st, const GskColArgs *cols = nullptr);  // G=8  R=5 W=8  40 rows,  64 thr
+cudaError_t gsk_local_launch_D(const GskLocalArgs &a, int e, cudaStream_t st, const GskColArgs *cols = nullptr);  // G=32 R=3 W=8  72 rows, 128 thr
+cudaError_t gsk_local_launch_E(const GskLocalArgs &a, int e, cudaStream_t st, const GskColArgs *cols = nullptr);  // G=32 R=4 W=8 112 rows, 128 thr

@@ -1,5 +1,5 @@
 // local_solve_B.cu — instantiates K3 for <G, R, W, RS, NT> = <4, 6, 4, 24, 128> (see local_solve.cuh)
 #include "local_solve.cuh"
-cudaError_t gsk_local_launch_B(const GskLocalArgs &a, int e, cudaStream_t st) {
-  return gsk_local::launch_cfg<4, 6, 4, 24, 128>(a, e, st);
+cudaError_t gsk_local_launch_B(const GskLocalArgs &a, int e, cudaStream_t st, const GskColArgs *cols) {
+  return cols ? gsk_local::launch_cfg<4, 6, 4, 24, 128, true>(a, *cols, e, st) : gsk_local::launch_cfg<4, 6, 4, 24, 128>(a, GskColArgs{}, e, st);
 }

@@ -603,6 +603,69 @@ def _solve_kriging(problem: EstimationProblem, solver: KrigingSolver, ctx, path_
     return georef({**mus, **sigmas}, pdomain)                           # krig.jl:163
 
 
+def _same_param(a, b) -> bool:
+    """Equal solver parameters: same value, or objects of one type with equal attributes (variograms, paths and
+    neighbourhoods compare by what they hold; closures only when identical)."""
+    if a is b:
+        return True
+    if type(a) is not type(b):
+        return False
+    if isinstance(a, np.ndarray):
+        return a.shape == b.shape and bool(np.all(a == b))
+    if isinstance(a, (tuple, list)):
+        return len(a) == len(b) and all(_same_param(x, y) for x, y in zip(a, b))
+    if hasattr(a, "__dict__") and not callable(a):
+        return vars(a).keys() == vars(b).keys() and all(_same_param(vars(a)[k], vars(b)[k]) for k in vars(a))
+    return bool(a == b)
+
+
+def krige_columns(problem: EstimationProblem, solver: KrigingSolver, ctx: Optional[_abi.Context] = None,
+                  path_order: bool = True) -> GeoTable:
+    """All variables of ``problem`` kriged in ONE library call (``gsk_krige_columns``): the neighbour search and the
+    factorisation of every target's system run once, each variable is one value column. Returns the columns `solve`
+    returns (`var` and `var_variance` per variable, in path order by default; units as `solve` gives them). The
+    variables must share their non-missing samples and have identical `KrigingSolver` parameters; otherwise a
+    ValueError names the first difference. The means agree with `solve`'s to rounding, not bit for bit."""
+    if not isinstance(solver, KrigingSolver):
+        raise _unsupported(f"krige_columns with {type(solver).__name__} (Kriging only)")
+    variables = list(problem.variables())
+    pdomain = problem.domain()
+    first = variables[0]
+    ref_params = solver.params(first)
+    ref_inds = None
+    for var in variables:
+        z = uadjust(problem.data().table[var])
+        _, missing = _split_missing(z.values if isinstance(z, Quantities) else z)
+        inds = np.flatnonzero(~missing)
+        if ref_inds is None:
+            ref_inds = inds
+        elif not np.array_equal(inds, ref_inds):
+            raise ValueError(f"krige_columns: {var} and {first} have different non-missing samples")
+        params = solver.params(var)
+        for key in ref_params:
+            if not _same_param(params.get(key), ref_params[key]):
+                raise ValueError(f"krige_columns: KrigingSolver parameter `{key}` of {var} differs from {first}'s")
+    preproc = preprocess(problem, solver)
+    pp = preproc[first]
+    local = pp["maxneighbors"] is not None
+    spec = _problem_spec(pp["samples"], pdomain, first, pp, local=local,
+                         order=_path_order(pdomain, pp["path"], path_order))
+    Z = np.column_stack([np.asarray(preproc[v]["samples"].table[v], dtype=np.float64) for v in variables])
+    mean, variance, nneigh = (ctx or default_context()).krige_columns(spec, Z, want_nneigh=True)
+    miss = nneigh < max(int(pp["minneighbors"]), 1) if local else np.zeros(len(variance), dtype=bool)
+    mus, sigmas = {}, {}
+    for j, var in enumerate(variables):
+        mu, sig = mean[:, j].copy(), variance.copy()
+        if miss.any():
+            mu, sig = np.ma.MaskedArray(mu, mask=miss), np.ma.MaskedArray(sig, mask=miss.copy())
+        unit = preproc[var]["unit"]
+        if unit is not NoUnits:
+            mu, sig = Quantities(mu, unit), Quantities(sig, unit ** 2)
+        mus[var] = mu
+        sigmas[f"{var}_variance"] = sig
+    return georef({**mus, **sigmas}, pdomain)
+
+
 def leave_one_out(data: GeoTable, solver: KrigingSolver, ctx: Optional[_abi.Context] = None) -> GeoTable:
     """Leave-one-out cross-validation (GeoStatsValidation's ``LeaveOneOut`` folds, each solved by ``solver``) as one
     library call per variable: row i of column `var` is sample i kriged at its own location from the other non-missing

@@ -150,8 +150,8 @@ typedef struct gsk_problem {
 
 typedef struct gsk_ctx gsk_ctx; /* opaque: one CUDA device, its stream, resident buffers */
 
-/* per-phase device times (CUDA events on the context stream) of the last gsk_execute/gsk_krige/gsk_krige_loo
- * (leave-one-out: ms_search includes the removal of each row's own index; on the global path ms_solve is the
+/* per-phase device times (CUDA events on the context stream) of the last gsk_execute/gsk_krige/gsk_krige_loo/
+ * gsk_krige_columns (columns: ms_solve includes the per-column epilogue; leave-one-out: ms_search includes the removal of each row's own index; on the global path ms_solve is the
  * pass over L⁻¹ that yields every row's leave-one-out residual and variance) */
 typedef struct gsk_timing {
   double ms_plan;    /* H2D of samples + bin build, or global assembly + factorisation */
@@ -186,6 +186,22 @@ GSK_API int gsk_krige(gsk_ctx *ctx, const gsk_problem *prob,
  * gsk_krige. The context holds no plan afterwards. */
 GSK_API int gsk_krige_loo(gsk_ctx *ctx, const gsk_problem *prob, double *mean_out, double *var_out,
                           int32_t *nneigh_out, int32_t *neigh_idx_out);
+
+/* Kriging of m value columns over one sample set: the search and the factorisation of every target's system run
+ * once and are applied to each column. Everything but the values behaves as in gsk_krige (domain, slab,
+ * target_order, support, estimator, neighbourhood, min_neighbors, flags, local/global switch); column j of
+ * mean_out is what gsk_krige computes with prob->values = column j, up to rounding (Simple Kriging:
+ * μ + Σ λᵢ (z_ij − μ)). Rows below min_neighbors are NaN in every column. prob->values must be NULL, n_cols >= 1,
+ * values non-NULL; GSK_FLAG_REUSE_PLAN is rejected, IDW / LWR are GSK_ERR_UNSUPPORTED. The local path solves
+ * [C F; Fᵀ 0][λ; ν] = [c; f] for the weights λ and Lagrange multipliers ν (rows below min_neighbors: λ = 0,
+ * ν = NaN); the global path applies the dual weights of each column. The context holds no plan afterwards. */
+GSK_API int gsk_krige_columns(gsk_ctx *ctx, const gsk_problem *prob,
+                              int32_t n_cols, const double *values,  /* n_samples × n_cols, row-major: values[i*n_cols + j] */
+                              double *mean_out,                      /* count × n_cols, row-major: mean_out[t*n_cols + j] */
+                              double *var_out,                       /* count (the variance does not depend on the values) */
+                              int32_t *nneigh_out, int32_t *neigh_idx_out,  /* optional, exactly as gsk_krige */
+                              double *weights_out,   /* optional, local path only: count × max_neighbors, 0-padded */
+                              double *lagrange_out); /* optional, local path only: count × nterms (OK 1, UK C(d+deg,deg), SK none) */
 
 /* ---- single-process multi-GPU convenience (a Julia host drives all GPUs of a box from one process):
  * the slab [target_first, target_first+target_count) is split into n_devices contiguous pieces, one host

@@ -191,6 +191,82 @@ function solve_b200(problem::EstimationProblem, solver::KrigingSolver; ctx=conte
 end
 
 """
+all variables of `problem` kriged in one gsk_krige_columns call: the search and the factorisation of every target's
+system run once, each variable is one value column. The variables must have the same non-missing samples and identical
+`KrigingSolver` parameters (an ArgumentError names the first difference). Returns the columns `solve_b200` returns
+(`var`, `var_variance` per variable, in path order); the means agree with `solve_b200`'s to rounding.
+"""
+function krigecolumns_b200(problem::EstimationProblem, solver::KrigingSolver; ctx=context())
+  pdata = data(problem); dtable = values(pdata); ddomain = domain(pdata); pdomain = domain(problem)
+  vars = Symbol[]; ps = []; zs = []
+  for covars in covariables(problem, solver), var in covars.names
+    push!(vars, var); push!(ps, covars.params[Set([var])])
+    push!(zs, uadjust(Tables.getcolumn(Tables.columns(dtable), var)))             # krig.jl:94
+  end
+  p = ps[1]
+  p.distance isa Euclidean || throw(ArgumentError("non-Euclidean `distance` is not supported by the B200 Kriging path"))
+  inds = findall(!ismissing, zs[1])                                                # krig.jl:97
+  isempty(inds) && throw(AssertionError("all samples of $(vars[1]) are missing, aborting..."))
+  for j in 2:length(vars)
+    findall(!ismissing, zs[j]) == inds ||
+      throw(ArgumentError("krigecolumns_b200: $(vars[j]) and $(vars[1]) have different non-missing samples"))
+    for f in propertynames(p)
+      isequal(getproperty(ps[j], f), getproperty(p, f)) ||
+        throw(ArgumentError("krigecolumns_b200: KrigingSolver parameter `$f` of $(vars[j]) differs from $(vars[1])'s"))
+    end
+  end
+  sdom = view(ddomain, inds)
+  estimator = GeoStatsSolvers.kriging_ui(pdomain, p.variogram, p.mean, p.degree, p.drifts)
+  searcher = GeoStatsSolvers.searcher_ui(sdom, p.maxneighbors, p.distance, p.neighborhood)
+  islocal = !isnothing(p.maxneighbors)
+  γ = estimator.γ
+  dim = embeddim(sdom); n = length(inds); m = length(vars)
+  X = [Float64[ustrip(coordinates(centroid(sdom, i))[d]) for i in 1:n] for d in 1:dim]
+  Z = Matrix{Float64}(undef, m, n)                      # column-major m × n = the ABI's row-major n × m
+  for j in 1:m
+    Z[j, :] .= Float64.(ustrip.(zs[j][inds]))
+  end
+  sup = support_offsets(pdomain, γ)
+  T = nelements(pdomain)
+  isgrid = pdomain isa CartesianGrid
+  P = isgrid ? [Float64[] for _ in 1:dim] : [Float64[ustrip(coordinates(centroid(pdomain, i))[d]) for i in 1:T] for d in 1:dim]
+  order = pathorder(pdomain, p.path)
+  tup(v, fill) = ntuple(d -> d <= length(v) ? v[d] : fill, 3)
+  ptrs(v) = ntuple(d -> d <= length(v) ? pointer(v[d]) : Ptr{Float64}(C_NULL), 3)
+  est, skmean, deg = estimator isa GeoStatsModels.SimpleKriging ? (Int32(0), Float64(ustrip(estimator.μ)), Int32(0)) :
+                     estimator isa GeoStatsModels.UniversalKriging ? (Int32(2), 0.0, Int32(maximum(estimator.exponents))) :
+                     estimator isa GeoStatsModels.OrdinaryKriging ? (Int32(1), 0.0, Int32(0)) :
+                     throw(ArgumentError("ExternalDriftKriging (`drifts`) is not supported by the B200 Kriging path"))
+  k = islocal ? Int32(maxneighbors(searcher)) : Int32(0)
+  radius = (islocal && searcher isa KBallSearch) ? Float64(ustrip(Meshes.radius(searcher.ball))) : NaN
+  M = Matrix{Float64}(undef, m, T); σ² = Vector{Float64}(undef, T); nn = Vector{Int32}(undef, T)
+  GC.@preserve X Z sup P M σ² nn order begin
+    prob = GskProblem(2, dim, n, ptrs(X), Ptr{Float64}(C_NULL),                  # values: the columns
+      isgrid ? tup(collect(Int64, size(pdomain)), 1) : (0, 1, 1),
+      isgrid ? tup(collect(Float64, ustrip.(coordinates(minimum(pdomain)))), 0.0) : (0.0, 0.0, 0.0),
+      isgrid ? tup(collect(Float64, ustrip.(spacing(pdomain))), 1.0) : (1.0, 1.0, 1.0),
+      isgrid ? 0 : T, ptrs(P), 0, -1, length(sup[1]), ptrs(sup),
+      variokind(γ), ustrip(range(γ)), ustrip(sill(γ)), ustrip(nugget(γ)), 1e-6,
+      est, skmean, deg, Int32(p.minneighbors), k, radius, UInt32(3),
+      isnothing(order) ? Ptr{Int64}(C_NULL) : pointer(order), Int32(0), 1.0, Int32(0))
+    check(ctx, ccall((:gsk_krige_columns, LIB), Cint,
+      (Ptr{Cvoid}, Ref{GskProblem}, Int32, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}, Ptr{Int32},
+       Ptr{Float64}, Ptr{Float64}),
+      ctx.handle, prob, Int32(m), Z, M, σ², nn, C_NULL, C_NULL, C_NULL))
+  end
+  miss = islocal ? nn .< max(p.minneighbors, 1) : falses(T)                       # krig.jl:213-214
+  varσ = ifelse.(miss, missing, σ²)
+  μs = []; σs = []
+  for j in 1:m
+    varμ = ifelse.(miss, missing, M[j, :])
+    u = elunit(zs[j])
+    push!(μs, vars[j] => (u == NoUnits ? varμ : varμ .* u))
+    push!(σs, Symbol(vars[j], "_variance") => (u == NoUnits ? varσ : varσ .* u^2))
+  end
+  georef((; μs..., σs...), pdomain)
+end
+
+"""
 leave-one-out cross-validation of `data` with `solver` (what GeoStatsValidation's `LeaveOneOut` computes by solving one
 fold per sample): per variable one gsk_krige_loo call; row i is sample i kriged at its own location from the other
 non-missing samples. Returns `var` and `var_variance` on the data domain in data order, `missing` where the value is
